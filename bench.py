@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py — fastq_info hot path throughput on B200 (BASELINE.json metric: FASTQ GB/s and reads/s validated).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--workload illumina_pe|illumina_se|longread]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--workload illumina_pe|illumina_se|longread] [--dump-outputs DIR]
 
 One step = one complete fastq_info job over synthetic input already resident in HBM.  Workloads (SURVEY.md §8d):
 
@@ -16,6 +16,8 @@ transcript (clean run included, at full size) is compared with the text the refe
 At N=1 the line also carries `also`: the 400 M-pair job streamed through one GPU (`illumina_pe_streamed`) and the command line on gzip
 operands against the reference binary, host inflate included (`gz_cli`).
 The reference arm times the unmodified reference binary (oracle/_ref/fastq_info, 1 thread — it has none) on a bounded sample.
+`--dump-outputs DIR` writes what the last timed step returned (the report and the transcript rendered from it) as DIR/<name>.npy,
+so that two builds can be compared output for output: the inputs are generated from fixed seeds.
 """
 import argparse
 import json
@@ -193,6 +195,26 @@ def _same(got, want, what, parity):
     return ok
 
 
+def dump_outputs(d, rep, transcript):
+    """The report of one job (include/fastq_gpu.h: fqg_report) and its rendered transcript as float64 .npy files under d.  Report
+    fields are 64-bit integers, which float64 holds exactly only below 2**53: each field is stored as the pair (high 32 bits, low 32
+    bits) along the last axis.  The transcript's text is stored as byte codes.  The error's header and name strings are left out (the
+    timed job raises no error)."""
+    import numpy as np
+    os.makedirs(d, exist_ok=True)
+    u64 = lambda xs: np.array([[(int(x) & KEY_NONE) >> 32, int(x) & 0xFFFFFFFF] for x in xs], dtype=np.float64)  # noqa: E731
+    e = rep.error
+    arrays = {"report_files": np.stack([u64([f.n_records, f.num_rds, f.min_rl, f.max_rl, f.min_qual, f.max_qual, f.sniff_format, f.color_space])
+                                        for f in rep.file]),  # per file: n_records num_rds min_rl max_rl min_qual max_qual sniff_format color_space
+              "report_index": u64([rep.mode, rep.n_index_entries, rep.n_index_left, rep.index_mem, rep.median_rl, *rep.reads_before_error]),
+              "report_error": u64([e.code, e.file, e.msg_file, e.chr, e.record, e.line, e.a, e.b, e.event_key]),
+              "exit_status": np.array([transcript[0]], dtype=np.float64),
+              "stdout": np.frombuffer(transcript[1].encode("latin-1"), dtype=np.uint8).astype(np.float64),
+              "stderr": np.frombuffer(transcript[2].encode("latin-1"), dtype=np.uint8).astype(np.float64)}
+    for name, arr in arrays.items():
+        np.save(os.path.join(d, name + ".npy"), arr)
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
@@ -205,7 +227,12 @@ def main():
     ap.add_argument("--no-e2e", action="store_true")
     ap.add_argument("--no-extras", action="store_true", help="N=1: skip the `also` runs (other configurations, the streamed 400 M-pair job)")
     ap.add_argument("--cpu-sample-reads", type=int, default=1_000_000, help="records (pairs) of the CPU baseline's sample")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the report and transcript of the last timed step as DIR/<name>.npy")
     a = ap.parse_args()
+    if a.steps < 1:
+        ap.error("--steps must be at least 1")
+    if a.dump_outputs and a.impl == "reference":
+        ap.error("--dump-outputs writes what our timed job computed: not available with --impl reference")
 
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
@@ -483,6 +510,8 @@ def main():
     # ---- parity of the timed job itself, at full size
     if rank == 0:
         tr = transcript_of(rep)
+        if a.dump_outputs:
+            dump_outputs(a.dump_outputs, rep if world == 1 else rep["report"], tr)
         if want_clean is not None:
             _same(tr, want_clean, "timed_job_transcript", parity)
         else:  # long reads: number of reads, length range and median from the generator's lengths; qualities 35..93 are `sanger`

@@ -103,6 +103,21 @@ def oracle_run_files(argv, cwd=GOLDEN):
     return oracle_run(argv, datas[0], datas[1])
 
 
+def have_ref(tool="fastq_info"):
+    return os.path.exists(os.path.join(ROOT, "oracle", "_ref", tool))
+
+
+def fuzz_golden(name):
+    """What the reference binaries returned on the seeded fuzz inputs of one test (tests/golden/fuzz/<name>.json, written by
+    tests/golden/make_fuzz_golden.py): the fuzz tests compare with it where the binaries are not built."""
+    path = os.path.join(GOLDEN, "fuzz", name + ".json")
+    if not os.path.exists(path):
+        import pytest
+        pytest.skip(f"neither the reference binaries (oracle/_ref) nor tests/golden/fuzz/{name}.json: run tests/golden/make_fuzz_golden.py where they are built")
+    with open(path) as fh:
+        return json.load(fh)
+
+
 def ref_run(argv, cwd=GOLDEN):
     """Run the unmodified reference binary (oracle/_ref) → (rc, stdout, stderr)."""
     p = subprocess.run([REF_BIN] + list(argv), cwd=cwd, capture_output=True)

@@ -1,7 +1,8 @@
 """fastq_filterpair (src/fastq_filterpair.c) behind fqg_filterpair_mem: file 1 through the index loop (validation, duplicate check), the
 records of both files delimited by the reader loop, names hashed and looked up in the index on the device, the reference's sequential
 bookkeeping (lookup-then-delete, seek counters, where its last loop starts) replayed on the host.  Against the committed transcripts of the
-reference's own binary (exit status, stdout, stderr, the three inflated output files) and, fuzzed, against the binary."""
+reference's own binary (exit status, stdout, stderr, the three inflated output files) and, fuzzed, against the binary (where it is
+not built, against its stored results for the same seeds)."""
 import ctypes
 import gzip
 import hashlib
@@ -14,7 +15,7 @@ import tempfile
 
 import pytest
 
-from _util import GOLDEN, ROOT, read_stream
+from _util import GOLDEN, ROOT, fuzz_golden, read_stream
 
 sys.path.insert(0, GOLDEN)
 from make_filterpair_golden import big_pair  # noqa: E402
@@ -104,36 +105,60 @@ def _fuzz_pair(rng):
     return a, b
 
 
-def _against_binary(seed, kind):
-    from fastq_utils_b200 import api
-    if not os.path.exists(REF):
-        pytest.skip("oracle/_ref/fastq_filterpair not built")
+def fuzz_runs(seed):
+    """seed -> 8 (argv, contents of a.fq, contents of b.fq)"""
     rng = random.Random(seed)
+    runs = []
+    for _ in range(8):  # (the reference takes 1.5 s per run: it clears a table of 100 000 001 buckets)
+        a, b = _fuzz_pair(rng)
+        runs.append((["a.fq", "b.fq", "p1.gz", "p2.gz", "up.gz"] + rng.choice([[], [], ["sorted"]]), a, b))
+    return runs
+
+
+def _digest(b):
+    return [len(b), hashlib.sha256(b).hexdigest()]
+
+
+def reference_result(seed):
+    """the reference binary on fuzz_runs(seed) -> per run [rc, stdout, stderr, created, (length, sha256) of the three inflated outputs
+    when it reported its counts, else None]"""
+    out = []
     with tempfile.TemporaryDirectory() as d:
-        for _ in range(8):  # (the reference takes 1.5 s per run: it clears a table of 100 000 001 buckets)
-            a, b = _fuzz_pair(rng)
+        for argv, a, b in fuzz_runs(seed):
             for nm, dta in (("a.fq", a), ("b.fq", b)):
                 with open(os.path.join(d, nm), "wb") as fh:
                     fh.write(dta)
-            argv = ["a.fq", "b.fq", "p1.gz", "p2.gz", "up.gz"] + rng.choice([[], [], ["sorted"]])
             for o in argv[2:5]:
                 if os.path.exists(os.path.join(d, o)):
                     os.unlink(os.path.join(d, o))
             pr = subprocess.run([REF] + argv, cwd=d, capture_output=True)
-            rc, out, err, created, bufs = api.filterpair(argv, a, b, _lib=_lib(kind))
-            assert (rc, out, err) == (pr.returncode, pr.stdout.decode("latin-1"), pr.stderr.decode("latin-1")), (argv, a, b)
-            assert created == all(os.path.exists(os.path.join(d, o)) for o in argv[2:5])
-            if "\nPaired: " in err:
-                for k, o in enumerate(argv[2:5]):
-                    assert bufs[k] == gzip.open(os.path.join(d, o), "rb").read(), (argv, k, a, b)
+            err = pr.stderr.decode("latin-1")
+            outs = [_digest(gzip.open(os.path.join(d, o), "rb").read()) for o in argv[2:5]] if "\nPaired: " in err else None
+            out.append([pr.returncode, pr.stdout.decode("latin-1"), err, all(os.path.exists(os.path.join(d, o)) for o in argv[2:5]), outs])
+    return out
 
 
-@pytest.mark.parametrize("seed", range(3))
+def _against_binary(seed, kind):
+    """against the reference binary where it is built, else against its stored results for the same seed"""
+    from fastq_utils_b200 import api
+    wants = reference_result(seed) if os.path.exists(REF) else fuzz_golden("filterpair_fuzz")[str(seed)]
+    for (argv, a, b), want in zip(fuzz_runs(seed), wants):
+        rc, out, err, created, bufs = api.filterpair(argv, a, b, _lib=_lib(kind))
+        assert [rc, out, err] == want[:3], (argv, a, b)
+        assert created == want[3]
+        if want[4] is not None:
+            assert [_digest(x) for x in bufs] == want[4], (argv, a, b)
+
+
+SEEDS_SIM, SEEDS_GPU = range(3), range(100, 102)
+
+
+@pytest.mark.parametrize("seed", SEEDS_SIM)
 def test_sim_filterpair_fuzz_against_binary(seed):
     _against_binary(seed, "sim")
 
 
 @pytest.mark.gpu
-@pytest.mark.parametrize("seed", range(100, 102))
+@pytest.mark.parametrize("seed", SEEDS_GPU)
 def test_gpu_filterpair_fuzz_against_binary(seed):
     _against_binary(seed, "gpu")

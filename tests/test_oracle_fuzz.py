@@ -1,16 +1,15 @@
 """Differential fuzz: oracle (CPU restatement) vs the unmodified reference binary (oracle/_ref/fastq_info).
 
-Seeded mutations of small FASTQ streams in all five modes; transcripts must be byte-identical.  Skipped when
-the reference binary has not been built (it is git-ignored but travels to the GPU box).
+Seeded mutations of small FASTQ streams in all five modes; transcripts must be byte-identical.  Where the reference binary is not
+built, the oracle is compared with the reference's transcripts of the same seeds (tests/golden/fuzz/oracle_fuzz.json).
 """
 import os
 import random
+import tempfile
 
 import pytest
 
-from _util import REF_BIN, oracle_run, ref_run
-
-pytestmark = pytest.mark.skipif(not os.path.exists(REF_BIN), reason="oracle/_ref/fastq_info not built")
+from _util import fuzz_golden, have_ref, oracle_run, ref_run
 
 NAMES = [
     lambda i, m: f"r{i}/{m}",
@@ -73,8 +72,8 @@ def render(rng, recs, style):
     return s.encode("latin-1")
 
 
-@pytest.mark.parametrize("seed", range(240))
-def test_fuzz_against_reference_binary(tmp_path, seed):
+def fuzz_case(seed):
+    """seed -> (argv, file a.fq, file b.fq or None)"""
     rng = random.Random(seed)
     style = rng.randrange(len(NAMES))
     n = rng.choice([0, 1, 2, 3, 5, 8, 13])
@@ -94,16 +93,33 @@ def test_fuzz_against_reference_binary(tmp_path, seed):
     nlstyle = "crlf" if rng.random() < 0.08 else "lf"
     d1 = render(rng, r1, nlstyle)
     d2 = render(rng, r2, nlstyle) if two else None
-    (tmp_path / "a.fq").write_bytes(d1)
     argv = {"single": [], "single_r": ["-r"], "pe": [], "pair": [], "pair_rs": ["-r", "-s"], "pair_s": ["-s"], "pair_r": ["-r"]}[mode]
     if rng.random() < 0.2: argv = ["-q"] + argv
     if rng.random() < 0.2: argv = ["-e"] + argv
     argv = argv + ["a.fq"]
     if two:
-        (tmp_path / "b.fq").write_bytes(d2)
         argv.append("b.fq")
     if mode == "pe":
         argv.append("pe")
-    want = ref_run(argv, cwd=str(tmp_path))
+    return argv, d1, d2
+
+
+def reference_result(seed):
+    """the reference binary on the files of fuzz_case(seed) -> (rc, stdout, stderr)"""
+    argv, d1, d2 = fuzz_case(seed)
+    with tempfile.TemporaryDirectory() as d:
+        open(os.path.join(d, "a.fq"), "wb").write(d1)
+        if d2 is not None:
+            open(os.path.join(d, "b.fq"), "wb").write(d2)
+        return ref_run(argv, cwd=d)
+
+
+SEEDS = range(240)
+
+
+@pytest.mark.parametrize("seed", SEEDS)
+def test_fuzz_against_reference_binary(seed):
+    argv, d1, d2 = fuzz_case(seed)
+    want = reference_result(seed) if have_ref() else tuple(fuzz_golden("oracle_fuzz")[str(seed)])
     got = oracle_run(argv, d1, d2)
     assert got == want, (argv, d1, d2)

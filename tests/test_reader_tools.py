@@ -6,11 +6,10 @@ import random
 
 import pytest
 
-from _util import ROOT, fqg_reader_tool, fqg_reader_tool_files, reader_golden, ref_reader_tool
+from _util import ROOT, fqg_reader_tool, fqg_reader_tool_files, fuzz_golden, have_ref, reader_golden, ref_reader_tool
 from test_oracle_fuzz import NAMES, make_file, mutate, render
 
 CASES = reader_golden()
-HAVE_REF = os.path.exists(os.path.join(ROOT, "oracle", "_ref", "fastq_num_reads"))
 
 
 def _check(c, kind, chunk):
@@ -36,12 +35,24 @@ def _fuzz_file(seed):
     return data
 
 
-@pytest.mark.skipif(not HAVE_REF, reason="needs the reference tools built by `make -C oracle ref-tools`")
-@pytest.mark.parametrize("seed", range(150))
-def test_sim_reader_tools_fuzz_against_reference(seed):
+FUZZ_TOOLS = ("fastq_num_reads", "fastq_not_empty")
+
+
+def reference_result(seed):
+    """the reference tools on _fuzz_file(seed) -> [(rc, stdout, stderr) of each of FUZZ_TOOLS]"""
     data = _fuzz_file(seed)
-    for tool in ("fastq_num_reads", "fastq_not_empty"):
-        want = ref_reader_tool(tool, data)
+    return [ref_reader_tool(tool, data) for tool in FUZZ_TOOLS]
+
+
+SEEDS = range(150)
+
+
+@pytest.mark.parametrize("seed", SEEDS)
+def test_sim_reader_tools_fuzz_against_reference(seed):
+    """against the reference tools where they are built (make -C oracle ref-tools), else against their stored transcripts"""
+    data = _fuzz_file(seed)
+    wants = reference_result(seed) if have_ref("fastq_num_reads") else [tuple(w) for w in fuzz_golden("reader_fuzz")[str(seed)]]
+    for tool, want in zip(FUZZ_TOOLS, wants):
         got = fqg_reader_tool(tool, ["a.fq"], data, chunk=[0, 0, 37, 512][seed % 4], kind="sim")
         assert got == want, (tool, seed, data[:200])
 

@@ -7,7 +7,7 @@ import tempfile
 
 import pytest
 
-from _util import GOLDEN, REF_BIN, fqg_run_stream, golden_transcripts, positional_files, read_stream, ref_run
+from _util import GOLDEN, fqg_run_stream, fuzz_golden, golden_transcripts, have_ref, positional_files, read_stream, ref_run
 
 CASES = golden_transcripts()
 
@@ -29,18 +29,26 @@ def test_sim_stream_matches_reference_transcript(idx):
     assert got[:3] == (c["rc"], c["stdout"], c["stderr"]), (c["argv"], piece)
 
 
-@pytest.mark.skipif(not os.path.exists(REF_BIN), reason="needs the reference binary (oracle/_ref)")
-@pytest.mark.parametrize("argv", [["-rs", "a.fq", "b.fq"], ["--", "a.fq"], ["-r", "--", "a.fq"], ["a.fq", "-r"], ["-s", "a.fq", "b.fq"], ["-e", "a.fq", "b.fq", "pe"],
-                                  ["-r", "-s", "a.fq", "nope.fq"], ["nope.fq", "b.fq"], ["a.fq", "nope.fq"], ["-q", "-e", "b.fq"]])
-def test_sim_operands_like_the_reference(argv):
-    """which words the reference treats as file 1 / file 2 (argv[1 + nopt], src/fastq_info.c:258-266): clustered options shift them"""
-    a = "".join(f"@r{i}/1\nACGT\n+\nIIII\n" for i in range(3)).encode()
-    b = "".join(f"@r{i}/2\nTTTT\n+\nFFFF\n" for i in range(2)).encode()
+OPERAND_ARGVS = [["-rs", "a.fq", "b.fq"], ["--", "a.fq"], ["-r", "--", "a.fq"], ["a.fq", "-r"], ["-s", "a.fq", "b.fq"], ["-e", "a.fq", "b.fq", "pe"],
+                 ["-r", "-s", "a.fq", "nope.fq"], ["nope.fq", "b.fq"], ["a.fq", "nope.fq"], ["-q", "-e", "b.fq"]]
+OPERAND_A = "".join(f"@r{i}/1\nACGT\n+\nIIII\n" for i in range(3)).encode()
+OPERAND_B = "".join(f"@r{i}/2\nTTTT\n+\nFFFF\n" for i in range(2)).encode()
+
+
+def reference_result(argv):
+    """the reference binary with files a.fq and b.fq of OPERAND_A / OPERAND_B -> (rc, stdout, stderr)"""
     with tempfile.TemporaryDirectory() as d:
-        open(os.path.join(d, "a.fq"), "wb").write(a)
-        open(os.path.join(d, "b.fq"), "wb").write(b)
-        want = ref_run(argv, cwd=d)
-    got = fqg_run_stream(argv, {"a.fq": a, "b.fq": b}, piece=64, kind="sim")
+        open(os.path.join(d, "a.fq"), "wb").write(OPERAND_A)
+        open(os.path.join(d, "b.fq"), "wb").write(OPERAND_B)
+        return ref_run(argv, cwd=d)
+
+
+@pytest.mark.parametrize("argv", OPERAND_ARGVS)
+def test_sim_operands_like_the_reference(argv):
+    """which words the reference treats as file 1 / file 2 (argv[1 + nopt], src/fastq_info.c:258-266): clustered options shift them;
+    against the binary where it is built, else against its stored transcripts"""
+    want = reference_result(argv) if have_ref() else tuple(fuzz_golden("stream_operands")[" ".join(argv)])
+    got = fqg_run_stream(argv, {"a.fq": OPERAND_A, "b.fq": OPERAND_B}, piece=64, kind="sim")
     assert got[:3] == want, (argv, got, want)
 
 

@@ -1,6 +1,7 @@
 """fastq_trim_poly_at (src/fastq_trim_poly_at.c) behind fqg_trim_poly_at_stream: records delimited on the device by the reader loop, the
 poly-A / poly-T scans evaluated there, the reference's line-buffer edits replayed on the host.  Against the committed transcripts of the
-reference's own binary (exit status, stdout, stderr, inflated output file) and, fuzzed, against the binary."""
+reference's own binary (exit status, stdout, stderr, inflated output file) and, fuzzed, against the binary (where it is not built,
+against its stored results for the same seeds)."""
 import ctypes
 import gzip
 import hashlib
@@ -13,7 +14,7 @@ import tempfile
 
 import pytest
 
-from _util import GOLDEN, ROOT, read_stream
+from _util import GOLDEN, ROOT, fuzz_golden, read_stream
 
 sys.path.insert(0, GOLDEN)
 from make_trim_golden import poly_100k  # noqa: E402
@@ -107,34 +108,56 @@ def _fuzz_file(rng):
     return data
 
 
-def _against_binary(seeds, kind):
-    from fastq_utils_b200 import api
-    if not os.path.exists(REF):
-        pytest.skip("oracle/_ref/fastq_trim_poly_at not built")
-    rng = random.Random(seeds)
+def fuzz_runs(seed):
+    """seed -> 40 (argv, contents of f.fq)"""
+    rng = random.Random(seed)
+    runs = []
+    for _ in range(40):
+        data = _fuzz_file(rng)
+        opts = rng.choice([[], ["--min_poly_at_len", "2"], ["--min_poly_at_len", "9", "--min_len", "0"], ["--min_len", "30"], ["--min_poly_at_len", "1", "--min_len", "3"]])
+        runs.append((opts + ["--file", "f.fq", "--outfile", "o.gz"], data))
+    return runs
+
+
+def _digest(b):
+    return [len(b), hashlib.sha256(b).hexdigest()]
+
+
+def reference_result(seed):
+    """the reference binary on fuzz_runs(seed) -> per run [rc, stdout, stderr, (length, sha256) of the inflated output or None]"""
+    out = []
     with tempfile.TemporaryDirectory() as d:
-        for _ in range(40):
-            data = _fuzz_file(rng)
-            opts = rng.choice([[], ["--min_poly_at_len", "2"], ["--min_poly_at_len", "9", "--min_len", "0"], ["--min_len", "30"], ["--min_poly_at_len", "1", "--min_len", "3"]])
+        o = os.path.join(d, "o.gz")
+        for argv, data in fuzz_runs(seed):
             with open(os.path.join(d, "f.fq"), "wb") as fh:
                 fh.write(data)
-            o = os.path.join(d, "o.gz")
             if os.path.exists(o):
                 os.unlink(o)
-            argv = opts + ["--file", "f.fq", "--outfile", "o.gz"]
             pr = subprocess.run([REF] + argv, cwd=d, capture_output=True)
-            got = api.trim_poly_at(argv, files={"f.fq": data}, _lib=_lib(kind))
-            assert (got[0], got[1], got[2]) == (pr.returncode, pr.stdout.decode("latin-1"), pr.stderr.decode("latin-1")), (argv, data)
-            if pr.returncode == 0:
-                assert got[4] == gzip.open(o, "rb").read(), (argv, data)
+            out.append([pr.returncode, pr.stdout.decode("latin-1"), pr.stderr.decode("latin-1"), _digest(gzip.open(o, "rb").read()) if pr.returncode == 0 else None])
+    return out
 
 
-@pytest.mark.parametrize("seed", range(12))
+def _against_binary(seed, kind):
+    """against the reference binary where it is built, else against its stored results for the same seed"""
+    from fastq_utils_b200 import api
+    wants = reference_result(seed) if os.path.exists(REF) else fuzz_golden("trim_fuzz")[str(seed)]
+    for (argv, data), want in zip(fuzz_runs(seed), wants):
+        got = api.trim_poly_at(argv, files={"f.fq": data}, _lib=_lib(kind))
+        assert [got[0], got[1], got[2]] == want[:3], (argv, data)
+        if want[0] == 0:
+            assert _digest(got[4]) == want[3], (argv, data)
+
+
+SEEDS_SIM, SEEDS_GPU = range(12), range(100, 104)
+
+
+@pytest.mark.parametrize("seed", SEEDS_SIM)
 def test_sim_trim_fuzz_against_binary(seed):
     _against_binary(seed, "sim")
 
 
 @pytest.mark.gpu
-@pytest.mark.parametrize("seed", range(100, 104))
+@pytest.mark.parametrize("seed", SEEDS_GPU)
 def test_gpu_trim_fuzz_against_binary(seed):
     _against_binary(seed, "gpu")

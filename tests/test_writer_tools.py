@@ -10,7 +10,7 @@ import tempfile
 
 import pytest
 
-from _util import GOLDEN, ROOT, fqg_reader_tool, read_stream
+from _util import GOLDEN, ROOT, fqg_reader_tool, fuzz_golden, have_ref, read_stream
 
 CASES = json.load(open(os.path.join(GOLDEN, "writer_transcripts.json")))
 
@@ -73,14 +73,29 @@ def _fuzz_file(rng):
     return data
 
 
-@pytest.mark.skipif(not os.path.exists(os.path.join(ROOT, "oracle", "_ref", "fastq_truncate")), reason="needs the reference tools (oracle/_ref)")
-@pytest.mark.parametrize("seed", range(120))
-def test_sim_writer_tools_fuzz_against_reference(seed):
+def fuzz_case(seed):
+    """seed -> (tool, argv, contents of a.fq)"""
     rng = random.Random(4200 + seed)
     data = _fuzz_file(rng)
     tool, argv = ("fastq_truncate", ["a.fq", str(rng.choice([0, 1, 2, 5, 100, -3]))]) if seed % 2 else ("fastq_filter_n", rng.choice([[], ["-n", "0"], ["-n", "20"], ["-n", "60"]]) + ["a.fq"])
+    return tool, argv, data
+
+
+def reference_result(seed):
+    """the reference tool on fuzz_case(seed) -> (rc, stdout, stderr)"""
+    tool, argv, data = fuzz_case(seed)
     with tempfile.TemporaryDirectory() as d:
         open(os.path.join(d, "a.fq"), "wb").write(data)
         p = subprocess.run([os.path.join(ROOT, "oracle", "_ref", tool)] + argv, cwd=d, capture_output=True)
-    want = (p.returncode, p.stdout.decode("latin-1"), p.stderr.decode("latin-1"))
+    return p.returncode, p.stdout.decode("latin-1"), p.stderr.decode("latin-1")
+
+
+SEEDS = range(120)
+
+
+@pytest.mark.parametrize("seed", SEEDS)
+def test_sim_writer_tools_fuzz_against_reference(seed):
+    """against the reference tools where they are built, else against their stored transcripts"""
+    tool, argv, data = fuzz_case(seed)
+    want = reference_result(seed) if have_ref("fastq_truncate") else tuple(fuzz_golden("writer_fuzz")[str(seed)])
     assert fqg_reader_tool(tool, argv, data, kind="sim") == want, (tool, argv, data)
