@@ -77,7 +77,6 @@ void FqEngine::reset() {
   seed_ = 0; finished_ = false; total0_set_ = false; total0_ = 0; fused_ok_ = !(cfg_.flags & FQG_FLAG_TWO_PASS);
   { const char* e = getenv("FQG_FUSED_MIN_BYTES"); fused_min_ = e ? (uint32_t)strtoul(e, nullptr, 10) : (1u << 20); } /* test hook */
   { const char* e = getenv("FQG_NO_LANES"); lanes_ok_ = !(e && *e && *e != '0'); }                                  /* test hook */
-  { const char* e = getenv("FQG_ROUTE_AFTER"); hook_after_ = e && *e && *e != '0'; } /* A/B: the chunk hook fires when the chunk is done (the routing kernels then have the GPU to themselves) instead of beside the next pass */
   { const char* e = getenv("FQG_TEST_WEAK_HASH"); if (e && *e && *e != '0') seed_ = FQ_SEED_WEAK; }                 /* test hook: 12-bit name hashes, so that equal hashes of different names are common */
   for (auto& m : mem_stats) m = 0;
   open_ = streaming_; add_depth_ = 0; open_dirty_ = false;
@@ -315,10 +314,10 @@ void FqEngine::lanes_prepare(int file, uint8_t* data, uint32_t n, uint32_t lead,
   }
   /* While every chunk so far is final and no bytes wait for the rest of their record, an accepted clean-data pass is final too: its
    * statistics go straight into the main set (a chunk the pass hands on leaves no trace in either set). */
-  L->direct = open_ && add_depth_ == 1 && F.pend_n == 0 && !open_dirty_ && !getenv("FQG_NO_DIRECT");
+  L->direct = open_ && add_depth_ == 1 && F.pend_n == 0 && !open_dirty_;
   if (L->direct) { a.stats = f_[target].stats; a.hist = f_[target].hist; a.stats_range = f_[file].stats; }
   L->launched = dev_->lanes_pass(a, &L->self_judged);
-  if (L->launched && hook_ && !hook_after_) { /* the pass is running: the caller routes the names of the chunks before this one beside it */
+  if (L->launched && hook_) { /* the pass is running: the caller routes the names of the chunks before this one beside it */
     in_beside_hook_ = true; L->hooked = true;
     try { hook_(hook_user_, file); } catch (...) { in_beside_hook_ = false; throw; }
     in_beside_hook_ = false;
@@ -441,7 +440,7 @@ bool FqEngine::try_fused_pass(int file, int b, bool last, uint32_t j0, uint64_t 
  * feed_device) and its pass is launched now, while the host still has chunk k's segment, name kernels and settling to do.  Only when
  * nothing can move that start: what is left behind the last record must be a plain partial record (no line gzgets would split). */
 void FqEngine::launch_ahead(int file, const FqBuffer& B, uint32_t j0, uint64_t g0_local) {
-  if (!next_.valid || next_.file != file || getenv("FQG_NO_AHEAD")) return;
+  if (!next_.valid || next_.file != file) return;
   next_.valid = false;
   FqFile& F = f_[file];
   if (hook_ && F.route_world == 0) return; /* a caller that packs the name descriptors of finished chunks from its hook wants this chunk's segment first */

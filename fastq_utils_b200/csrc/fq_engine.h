@@ -143,7 +143,6 @@ class FqEngine {
   FqSlot* slots_ = nullptr; uint64_t table_cap_ = 0; uint64_t table_names_ = 0;
   uint32_t seed_ = 0;
   fqg_chunk_hook hook_ = nullptr; void* hook_user_ = nullptr;
-  bool hook_after_ = false;                 /* never call the hook beside a running pass */
   bool hook_fired_ = false;                 /* the chunk being fed has called the hook already */
   bool in_beside_hook_ = false;             /* the hook runs while a clean-data pass occupies the main stream */
   unsigned long long* route_cursors_ = nullptr; /* device: FQ_SHARD_MAX_SRC per-owner tuple counts of the round being packed */

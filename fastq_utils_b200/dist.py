@@ -44,8 +44,7 @@ class ShardedFastqInfo:
         # path only — the lines of a range do not say whether its first record is a first or a second mate).  MODE_SORTED_PAIR is NOT
         # sharded: file 2 would have to be cut by record index, not by byte offset (SURVEY.md §8e), which byte ranges do not give.  The
         # ranks' ranges are gathered on rank 0, whose engine runs the loop (at most 64 GiB in all); every rank gets the result.
-        # FQG_GATHER_INTERLEAVED=1 takes that way for interleaved files too (A/B).
-        self.gathered = mode == api.MODE_SORTED_PAIR or (mode == api.MODE_INTERLEAVED and os.environ.get("FQG_GATHER_INTERLEAVED", "0") not in ("", "0"))
+        self.gathered = mode == api.MODE_SORTED_PAIR
         self.lines_per_step = 8 if mode == api.MODE_INTERLEAVED else 4  # a range starts where a loop iteration starts
         self.mode = mode
         self.rank = dist.get_rank() if dist.is_initialized() else 0
@@ -61,27 +60,22 @@ class ShardedFastqInfo:
         if self.world > 1 and dist.get_backend() != "gloo":
             import datetime
             self._cpu_group = dist.new_group(backend="gloo", timeout=datetime.timedelta(seconds=int(os.environ.get("FQG_GLOO_TIMEOUT_S", "120"))))  # a rank that died must not hang the others for half an hour
-        self.pipeline = os.environ.get("FQG_NO_PIPELINE", "0") in ("", "0")
-        # pipelined rounds over peer memory (CUDA IPC) instead of all-to-all exchanges: the default on GPUs, FQG_P2P=0 turns it off;
-        # FQG_P2P=1 asks for it on CPU tensors too (the gloo tests: the stand-in device maps shared memory between the ranks)
+        # routing rounds over peer memory (CUDA IPC) instead of all-to-all exchanges: the default on GPUs.  Test hooks: FQG_P2P=0 runs
+        # the exchanges (the fallback when a peer cannot be mapped) on GPUs; FQG_P2P=1 runs peer memory on CPU tensors (the gloo tests:
+        # the stand-in device maps shared memory between the ranks)
         self.p2p = os.environ.get("FQG_P2P", "1" if self.tdev.type == "cuda" else "0") not in ("", "0")
-        # the copy engines move the packed regions; FQG_P2P_STORES=1: the pack kernel stores into the owners' arenas itself (A/B)
-        self.p2p_stores = os.environ.get("FQG_P2P_STORES", "0") not in ("", "0")
-        # FQG_NCCL_GATHER=0: the small gathers over gloo (A/B)
-        self._nccl_gather = (self.world > 1 and self.tdev.type == "cuda" and dist.get_backend() == "nccl" and os.environ.get("FQG_NCCL_GATHER", "1") not in ("", "0"))
+        self._nccl_gather = self.world > 1 and self.tdev.type == "cuda" and dist.get_backend() == "nccl"
         self._gbuf = None
-        self._owner_beside = int(os.environ.get("FQG_OWNER_BESIDE", "0") or 0)  # (A/B) 1: the owner's kernels beside the running pass, 2: the inserts only
-        # One copy stream per peer for the regions of a round (FQG_COPY_LANES=0: all on the side stream).  Measured on 8 B200s: 43.3 ms
-        # per job with one stream — seven copies of 60 MB one after the other take longer than the pass they should hide behind —
-        # 38.8 ms with seven; with four ranks no difference (34.2 / 34.5 ms).
-        self._copy_lanes = max(0, min(7, int(os.environ.get("FQG_COPY_LANES", str(self.world - 1)) or 0)))
-        self._pending_insert = None
+        # One copy stream per peer for the regions of a round.  Measured on 8 B200s: 43.3 ms per job with one stream — seven copies
+        # of 60 MB one after the other take longer than the pass they should hide behind — 38.8 ms with seven; with four ranks no
+        # difference (34.2 / 34.5 ms).
+        self._copy_lanes = min(7, self.world - 1)
         self._arena, self._peer, self._arena_failed, self._p2p_ok, self._stage, self._zero = None, None, False, False, None, None
-        self.rounds_done = 0  # routing rounds of the last pipelined run (tests, bench)
+        self.rounds_done = 0  # routing rounds of the last run (tests, bench)
         self._plan, self._job, self._flagvals = None, 0, None
         self.gathered_jobs = 0  # feeds that sent every range to rank 0 (tiny inputs, a NUL-led header line, the sorted-pair mode)
         self.exact_reruns = 0  # jobs the speculative / pipelined path handed to the exact path (tests)
-        self.host_ms = {"pack": 0.0, "barrier": 0.0}  # host time inside the peer-memory rounds, accumulated
+        self.host_ms = {"pack": 0.0}  # host time inside the peer-memory rounds, accumulated
         self.phase_ms = {}  # host wall time of the phases of run_device, accumulated over jobs (bench.py reports them)
 
     def route_description(self):
@@ -212,36 +206,16 @@ class ShardedFastqInfo:
         sn = self._gather(sn)[0]
         if sn[0] >= 0:
             ctx.set_sniff(f, sn[0], sn[1])
-        # head of range r+1 travels to rank r
-        head, reqs = None, []
-        if W > 1:
-            if r > 0 and cut[r] > 0:
-                view = _as_tensor(ptr, cut[r], self.tdev)
-                reqs.append(dist.isend(view, r - 1))
-                self._keep.append(view)
-            if r < W - 1 and cut[r + 1] > 0:
-                head = torch.zeros(cut[r + 1] + 64, dtype=torch.uint8, device=self.tdev)
-                reqs.append(dist.irecv(head[:cut[r + 1]], r + 1))
-            for q in reqs:
-                q.wait()
-            if reqs:
-                self._sync()  # the library reads the head on its own stream
         ctx.set_stream_start(f, skip[r], firstrec[r])
-        if last_rank:
-            ctx.feed_device(f, ptr, nbytes, last=True)
-        else:
-            ctx.feed_device(f, ptr, nbytes, last=False)
-            if head is not None:
-                ctx.feed_device(f, head.data_ptr(), cut[r + 1], last=True)
-                self._keep.append(head)
-            else:
-                ctx.feed(f, b"", last=True)
+        self._feed_range(f, ptr, nbytes, cut)
         expected = (lfs + virt - skip[r] + (skip[r + 1] if r < W - 1 else 0)) // 4
         return expected, total_records
 
-    def _first_line_ends(self, ptr, nbytes, k):
-        """ends (offsets behind the line feed) of the first k lines of this rank's range, KEY_NONE where the range has fewer"""
-        want, ends = 1 << 14, []
+    def _head_line_ends(self, ptr, nbytes, k, enough=None, limit=None):
+        """Ends (offsets behind the line feed) of the first k lines of this rank's range, fewer where the window has fewer, and the
+        window's bytes.  The window starts at 16 KiB and grows sixteenfold until `enough(head, ends)` holds (by default: k ends were
+        found), it holds the whole range, or it has reached `limit` bytes."""
+        want = 1 << 14
         while True:
             n = min(nbytes, want)
             head = bytes(_as_tensor(ptr, n, self.tdev).cpu().numpy())
@@ -251,33 +225,26 @@ class ShardedFastqInfo:
                 if pos < 0:
                     break
                 ends.append(pos + 1)
-            if len(ends) == k or n == nbytes:
-                return ends + [KEY_NONE] * (k - len(ends))
+            if (enough(head, ends) if enough else len(ends) == k) or n == nbytes or (limit and want >= limit):
+                return head, ends
             want *= 16
 
-    def _guess_phase(self, ptr, nbytes, want=1 << 14):
+    def _first_line_ends(self, ptr, nbytes, k):
+        """ends of the first k lines of this rank's range, KEY_NONE where the range has fewer"""
+        ends = self._head_line_ends(ptr, nbytes, k)[1]
+        return ends + [KEY_NONE] * (k - len(ends))
+
+    def _guess_phase(self, ptr, nbytes):
         """Line class (0 header, 1 sequence, 2 plus, 3 quality) of the line this range starts in, from the range's own first lines:
         a complete line that is exactly "+" is a plus line.  Returns (ok, class, ends of the first four lines, ends with LF, bytes
         per record over the first complete records, raw length of the first complete sequence line)."""
         if nbytes < 4096:
             return (False, 0, [KEY_NONE] * 4, True, 0.0, 0, b"")
-        k = min(nbytes, want)
-        head = bytes(_as_tensor(ptr, k, self.tdev).cpu().numpy())
+        # long lines: the window grows to 256 KiB (short reads are answered by the first 16 KiB)
+        head, ends = self._head_line_ends(ptr, nbytes, 64, enough=lambda h, e: len(e) >= 5 and _plus_line_class(h, e) is not None, limit=1 << 18)
         last = bytes(_as_tensor(ptr + nbytes - 1, 1, self.tdev).cpu().numpy())
-        ends, pos = [], -1
-        while len(ends) < 64:
-            pos = head.find(b"\n", pos + 1)
-            if pos < 0:
-                break
-            ends.append(pos + 1)
-        cls = None
-        for i in range(1, len(ends)):  # line i = head[ends[i-1]:ends[i]-1], complete
-            if ends[i] - ends[i - 1] == 2 and head[ends[i - 1]] == 0x2B:
-                cls = (2 - i) % 4
-                break
+        cls = _plus_line_class(head, ends)
         if cls is None or len(ends) < 5:
-            if want < (1 << 18) and nbytes > want:  # long lines: look further (short reads are answered by the first 16 KiB)
-                return self._guess_phase(ptr, nbytes, 1 << 18)
             return (False, 0, [KEY_NONE] * 4, last == b"\n", 0.0, 0, b"")
         k = (len(ends) - 1) // 4
         seq = next(ends[i] - ends[i - 1] for i in range(1, 5) if (cls + i) % 4 == 1)
@@ -305,7 +272,8 @@ class ShardedFastqInfo:
             line = first[1:first.index(b"\n")] if b"\n" in first else first[1:]
             name = line.split(b" ")[0] if self._sniff[0][0] == 1 else line
             units = max(1, -(-(len(name) + 3) // 16))
-        nb = self.ctx.route_blocks() if (self.p2p and not self.p2p_stores and os.environ.get("FQG_ROUTE_IN_PASS", "1") not in ("", "0")) else 0
+        # (test hook: FQG_ROUTE_IN_PASS=0 takes mode `pack` on GPUs, the mode of the stand-in device, whose pass routes nothing)
+        nb = self.ctx.route_blocks() if (self.p2p and os.environ.get("FQG_ROUTE_IN_PASS", "1") not in ("", "0")) else 0
         tiny = os.environ.get("FQG_TEST_SLOT_CAP")  # test hook: regions far too small, so that the overflow path is taken
         plan, base = [], FLAG_AREA
         self._job += 1
@@ -349,7 +317,7 @@ class ShardedFastqInfo:
         first plus line (`info`: the ranks' guesses, gathered).  A wrong guess cannot go unnoticed on a valid file (a sequence line
         lands where a header or a plus line is expected), so any error afterwards simply sends the whole job through the exact path."""
         W, r, ctx = self.world, self.rank, self.ctx
-        skip, cut = [0] * W, [0] * (W + 1)
+        skip, cut = [0] * W, [0] * W
         for i in range(1, W):
             cls0, prev_lf = info[i][1], info[i - 1][3]
             skip[i] = 0 if (prev_lf and cls0 == 0) else ((4 - cls0) % 4 or 4)
@@ -357,20 +325,6 @@ class ShardedFastqInfo:
         sn = self._sniff[f]
         if sn[0] >= 0:
             ctx.set_sniff(f, sn[0], sn[1])
-        head, reqs = None, []
-        if r > 0 and cut[r] > 0:
-            view = _as_tensor(ptr, cut[r], self.tdev)
-            reqs.append(dist.isend(view, r - 1))
-            self._keep.append(view)
-        if r < W - 1 and cut[r + 1] > 0:
-            head = torch.zeros(cut[r + 1] + 64, dtype=torch.uint8, device=self.tdev)
-            reqs.append(dist.irecv(head[:cut[r + 1]], r + 1))
-        _dbg(f"rank {r} file {f} seam exchange, {len(reqs)} requests")
-        for q in reqs:
-            q.wait()
-        if reqs:
-            self._sync()  # the library reads the head on its own stream
-        _dbg(f"rank {r} file {f} seam exchange done")
         ctx.set_stream_start(f, skip[r], 0)  # record numbers inside the range: they only matter when something is wrong
         ctx.set_line_hint(f, info[r][5])  # a range that starts inside the file never sees the first record's sequence line
         if routed:
@@ -382,7 +336,7 @@ class ShardedFastqInfo:
             ctx.set_chunk_hook(self._on_chunk)
         t0 = time.perf_counter()
         try:
-            self._feed_range(f, ptr, nbytes, head, cut[r + 1] if r < W - 1 else 0)
+            self._feed_range(f, ptr, nbytes, cut)
         finally:
             self.host_ms["feed"] = self.host_ms.get("feed", 0.0) + (time.perf_counter() - t0) * 1e3
             if routed:
@@ -399,17 +353,32 @@ class ShardedFastqInfo:
                 self._route_round(True)
             self.rounds_done += pl["round"]
 
-    def _feed_range(self, f, ptr, nbytes, head, head_n):
-        """This rank's range, then the head of the next range (the rest of the record its end cut)."""
+    def _feed_range(self, f, ptr, nbytes, cut):
+        """The seam between two byte ranges, then the feed.  cut[i]: bytes of range i in front of its first record start (the rest
+        of the record the end of range i-1 cut).  This rank sends its own to rank r-1, receives those of range r+1 and feeds its
+        range followed by them."""
         W, r, ctx = self.world, self.rank, self.ctx
-        cut = {r + 1: head_n}
+        head, reqs = None, []
+        if r > 0 and cut[r] > 0:
+            view = _as_tensor(ptr, cut[r], self.tdev)
+            reqs.append(dist.isend(view, r - 1))
+            self._keep.append(view)
+        if r < W - 1 and cut[r + 1] > 0:
+            head = torch.zeros(cut[r + 1] + 64, dtype=torch.uint8, device=self.tdev)
+            reqs.append(dist.irecv(head[:cut[r + 1]], r + 1))
+            self._keep.append(head)
+        _dbg(f"rank {r} file {f} seam exchange, {len(reqs)} requests")
+        for q in reqs:
+            q.wait()
+        if reqs:
+            self._sync()  # the library reads the head on its own stream
+        _dbg(f"rank {r} file {f} seam exchange done")
         if r == W - 1:
             ctx.feed_device(f, ptr, nbytes, last=True)
         else:
             ctx.feed_device(f, ptr, nbytes, last=False)
             if head is not None:
                 ctx.feed_device(f, head.data_ptr(), cut[r + 1], last=True)
-                self._keep.append(head)
             else:
                 ctx.feed(f, b"", last=True)
 
@@ -447,54 +416,61 @@ class ShardedFastqInfo:
         t1 = time.perf_counter()
         for d in range(W):
             o = (r + d) % W
-            dst = (self._arena[0] if o == r else self._peer[o]) + off
-            lane = 0 if (d == 0 or not self._copy_lanes) else 1 + (d - 1) % self._copy_lanes  # (FQG_COPY_LANES: the peers' regions on copy streams side by side)
-            if have:
-                self.ctx.side_copy_lane(lane, dst, st + (o * 2 + j % 2) * region, region)
-            else:
-                self.ctx.side_copy_lane(lane, dst, self._zero.data_ptr(), 16)
-            self._send_flag(o, f, j, lane)
+            src, n = (st + (o * 2 + j % 2) * region, region) if have else (self._zero.data_ptr(), 16)
+            self._send_region(o, off, src, n, f, j, lane=0 if d == 0 else 1 + (d - 1) % self._copy_lanes)  # (the peers' regions on copy streams side by side)
         self.ctx.side_mark()
         self.host_ms["pack"] += (time.perf_counter() - t1) * 1e3
         # The owner's kernel waits for its sources on the device (their flag words).  It takes the whole device between two passes:
         # behind the pass that is running now (launched ahead), in front of the next one.  Squeezed in beside a pass (one block
-        # per SM, FQG_OWNER_BESIDE=1) it was measured at a quarter of its speed, and the pass lost a third of its own.
-        between = beside and not (self._owner_beside == 1 or (self._owner_beside == 2 and f == 0))
-        if between:
+        # per SM) it was measured at a quarter of its speed, and the pass lost a third of its own.
+        if beside:
             self.shard.order_after(True, ctx, False)
-        self._owner_round(self._arena[0] + pl["base"] + j * W * region, region, pl["nblocks"], pl["stride"], pl["units"], f, beside and not between, flag_round=j)
-        if between and j + 2 < pl["rounds"]:  # (the last rounds have no pass behind them that would have to wait: the next file starts at once)
+        self._owner_round(self._arena[0] + pl["base"] + j * W * region, region, pl["nblocks"], pl["stride"], pl["units"], f, False, flag_round=j)
+        if beside and j + 2 < pl["rounds"]:  # (the last rounds have no pass behind them that would have to wait: the next file starts at once)
             ctx.order_after(False, self.shard, True)
         pl["round"] += 1
 
     def _left_round(self):
         """After the last chunk of a file, mode `pass`: what the per-record kernels validated (the seams between byte ranges, a short
         last chunk) has name descriptors; one packed round takes them to their owners.  Then every round of the file lands."""
-        W, r, f = self.world, self.rank, self._cur
+        f = self._cur
         pl = self._plan[f]
-        region, cap = pl["left_region"], pl["left_stride"]
         if os.environ.get("FQG_DEBUG_ROUTE"):
-            _dbg(f"rank {r} file {f} left round, names left {self.ctx.names_new(f)}")
-        # (the pack kernel below runs on the side stream, behind the copies out of the staging regions it overwrites: fqg_side_mark
-        # of the last round joined the copy lanes into that stream)
+            _dbg(f"rank {self.rank} file {f} left round, names left {self.ctx.names_new(f)}")
+        # (the pack kernel runs on the side stream, behind the copies out of the staging regions it overwrites: fqg_side_mark of the
+        # last round joined the copy lanes into that stream)
+        self._packed_round(f, pl["left_base"], pl["left_region"], pl["left_stride"], pl["units"], pl["rounds"], False)
+        self.ctx.side_mark()  # the next file's first pass writes into the staging regions: behind these copies
+
+    def _packed_round(self, f, base, region, cap, units, flag_round, beside):
+        """One round of names packed by the pack kernel (mode `pack`, and the left round of mode `pass`), over peer memory: the
+        region of every owner is `region` bytes at base + (source rank) * region in the owner's arena.  The pack kernel writes this
+        rank's own region straight into its arena and the others into staging, the copy engines move those to their owners with a
+        flag word behind each, and this rank's index shard takes the round (beside the running pass if `beside`).  The pack kernel
+        runs on the side stream, behind the copies of the round before out of the staging regions it overwrites.  (Stores from the
+        pack kernel straight into the peers' arenas were as fast with two ranks but slowed every pass threefold at eight: 5.9 M
+        remote stores per round and rank.)"""
+        W, r = self.world, self.rank
+        off = base + r * region
         st = self._stage.data_ptr()
-        off = pl["left_base"] + r * region
-        self.ctx.names_pack_slots(f, [self._arena[0] + off if o == r else st + o * region for o in range(W)], cap, pl["units"])
+        t0 = time.perf_counter()
+        self.ctx.names_pack_slots(f, [self._arena[0] + off if o == r else st + o * region for o in range(W)], cap, units)
         for d in range(W):
             o = (r + d) % W
-            if o != r:
-                self.ctx.side_copy(self._peer[o] + off, st + o * region, region)
-            self._send_flag(o, f, pl["rounds"])
-        self.ctx.side_mark()  # the next file's first pass writes into the staging regions: behind these copies
-        self._owner_round(self._arena[0] + pl["left_base"], region, 1, cap, pl["units"], f, False, flag_round=pl["rounds"])
+            self._send_region(o, off, None if o == r else st + o * region, region, f, flag_round)
+        self.host_ms["pack"] += (time.perf_counter() - t0) * 1e3
+        self._owner_round(self._arena[0] + base, region, 1, cap, units, f, beside, flag_round=flag_round)
 
     def _flag_off(self, f, j):
         return 8 * ((f * FLAG_ROUNDS + j) * self.world)
 
-    def _send_flag(self, o, f, j, lane=0):
-        """behind the bytes of round j for owner o (same stream of copies): the word that tells o's kernel they are there"""
-        dst = (self._arena[0] if o == self.rank else self._peer[o]) + self._flag_off(f, j) + 8 * self.rank
-        self.ctx.side_copy_lane(lane, dst, self._flagvals.data_ptr() + 8 * j, 8)
+    def _send_region(self, o, off, src, n, f, j, lane=0):
+        """n bytes from src to `off` in owner o's arena (src None: nothing to copy), then, behind them on the same copy stream, the flag
+        word of round j that tells o's kernel they are there"""
+        arena = self._arena[0] if o == self.rank else self._peer[o]
+        if src is not None:
+            self.ctx.side_copy_lane(lane, arena + off, src, n)
+        self.ctx.side_copy_lane(lane, arena + self._flag_off(f, j) + 8 * self.rank, self._flagvals.data_ptr() + 8 * j, 8)
 
     def _ensure_arena(self, need):
         """Peer-writable receive memory (CUDA IPC over NVLink): `need` bytes on every rank, mapped by every other rank.  Collective;
@@ -547,39 +523,6 @@ class ShardedFastqInfo:
         self._arena, self._peer = (ptr, size), peers
         return True
 
-    def _route_round_p2p(self, final):
-        """One routing round over peer memory, mode `pack`.  The names of this round are packed by owner next to the data and the
-        copy engines move each region into its owner's arena (CUDA IPC over NVLink): no exchange kernel needs SMs of its own, and
-        the pass keeps the memory system to itself (letting the pack kernel store into the peers' arenas directly, FQG_P2P_STORES=1,
-        is as fast with two ranks but slowed every pass threefold at eight: 5.9 M remote stores per round and rank).  A host barrier
-        says that every source's round has landed; it is passed in the NEXT round, a whole pass later, so nobody waits long; then
-        the owner inserts (file 1: claims) the round beside the running pass.  Pack first, insert second: both want the one block
-        slot per SM that the pass leaves free."""
-        W, r, f = self.world, self.rank, self._cur
-        pl = self._plan[f]
-        cap, units, stride = pl["stride"], pl["units"], pl["region"]
-        off = pl["base"] + pl["round"] * W * stride
-        t0 = time.perf_counter()
-        copies = []
-        if self.p2p_stores:
-            self.ctx.names_pack_slots(f, [self._peer[o] + off + r * stride for o in range(W)], cap, units)
-        else:
-            st = self._stage.data_ptr()
-            # (same stream as the copies of the round before: the pack overwrites the staging buffer after they have read it, and
-            # its completion says that they are done)
-            self.ctx.names_pack_slots(f, [self._arena[0] + off + r * stride if o == r else st + o * stride for o in range(W)], cap, units)
-            copies = [(self._peer[(r + d) % W] + off + r * stride, st + ((r + d) % W) * stride) for d in range(1, W)]
-        t1 = time.perf_counter()
-        for dst, src in copies:
-            self.ctx.side_copy(dst, src, stride)
-        for o in range(W):
-            self._send_flag(o, f, pl["round"])
-        self.host_ms["pack"] += (t1 - t0) * 1e3
-        # pack first, insert second (both want the one block slot per SM that the pass leaves free); the owner's kernel waits on the
-        # device for its sources' flag words: no host barrier
-        self._owner_round(self._arena[0] + off, stride, 1, cap, units, f, not final, flag_round=pl["round"])
-        pl["round"] += 1
-
     def _owner_round(self, regions_ptr, region_bytes, nblocks, stride, units, f, beside, flag_round=None):
         """this rank's index shard takes a round: file 1's names are inserted, file 2's claim them"""
         kw = {}
@@ -591,12 +534,15 @@ class ShardedFastqInfo:
             self.shard.shard_claim_slots(regions_ptr, self.world, region_bytes, nblocks, stride, beside=beside, units=units, **kw)
 
     def _route_round(self, final):
-        """Pack the names that were not routed yet into one fixed-capacity region per owner, start their exchange and hand the
-        rounds whose exchange has finished to this rank's index shard (beside the running pass unless this is the last round)."""
-        if self._p2p_ok:
-            return self._route_round_p2p(final)
+        """Modes `pack` and `a2a`: pack the names that were not routed yet into one fixed-capacity region per owner.  Over peer memory
+        the round is one packed round; otherwise start their exchange and hand the rounds whose exchange has finished to this rank's
+        index shard.  Either way the shard takes them beside the running pass unless this is the last round."""
         W, f = self.world, self._cur
         pl = self._plan[f]
+        if self._p2p_ok:
+            self._packed_round(f, pl["base"] + pl["round"] * W * pl["region"], pl["region"], pl["stride"], pl["units"], pl["round"], not final)
+            pl["round"] += 1
+            return
         units = pl["units"]
         mx = max(self._gather(self.ctx.names_new(f)))
         per = -(-mx // W)
@@ -692,10 +638,10 @@ class ShardedFastqInfo:
         pair = self.mode == api.MODE_INDEX_PAIR
         allr = None  # every rank's report, once gathered
         again = dict(name=name, ptr2=ptr2, nbytes2=nbytes2, name2=name2, empty_ok=empty_ok, no_enc_ok=no_enc_ok, _exact=True)
-        routed = self.shard is not None and self.pipeline
+        routed = self.shard is not None
         self.rounds_done = 0
         # (a world of one takes the same path when it has an index shard: the single-GPU tests of the pipelined routing)
-        speculative = (not _exact) and (W > 1 or routed) and (routed or not pair) and self.mode != api.MODE_INTERLEAVED
+        speculative = (not _exact) and (W > 1 or routed) and self.mode != api.MODE_INTERLEAVED
         files = [(0, ptr, nbytes)] + ([(1, ptr2, nbytes2)] if pair else [])
         if speculative:
             # every rank guesses the line phase of its ranges from their own first lines; rank 0, which holds the first record of each
@@ -747,10 +693,6 @@ class ShardedFastqInfo:
                     raise RuntimeError("the chunk hook of another rank failed (its exception is raised there)")
             else:
                 bad = any(self._gather(rep.error.code != 0 or cut_short))  # every rank takes the same turn: the steps below are collective
-            if not bad and self.shard is not None and not routed:
-                meta, blob, ms, bs = self._route_names(0, with_bytes=False)
-                self.shard.shard_insert(meta.data_ptr(), ms[-1], 0, ms, bs)
-                bad = any(self._gather(self.shard.shard_result()[3] > 0))
             if bad:
                 self.exact_reruns += 1
                 return self.run_device(ptr, nbytes, **again)  # an error, a duplicate name or a wrong guess: the exact path decides
@@ -899,6 +841,15 @@ def _local_hist(ctx, f0, f1):
     if not (lo <= hi < MAX_READ_LENGTH):
         return None
     return (lo, ctx.hist_range(0, lo, hi).tolist())
+
+
+def _plus_line_class(head, ends):
+    """line class of the range's first line, from the first complete line (line i = head[ends[i-1]:ends[i]-1]) that is exactly "+";
+    None without one"""
+    for i in range(1, len(ends)):
+        if ends[i] - ends[i - 1] == 2 and head[ends[i - 1]] == 0x2B:
+            return (2 - i) % 4
+    return None
 
 
 def _dbg(msg):

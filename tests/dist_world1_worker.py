@@ -21,12 +21,12 @@ big = [f"@M0:1:FC:1:11:{i}:{i * 7} 1:N:0:AC\n{'ACGTN' * (3 + i % 5)}\n+\n{'F' * 
 dup = list(big); dup[3900] = dup[17]
 nul = list(big); nul[1500] = "\x00" + nul[1500]
 bad = list(big); bad[3000] = bad[3000].replace("ACGTN", "ACXTN", 1)
-HOOKS = ("FQG_MAX_CHUNK_BYTES", "FQG_P2P", "FQG_TEST_WEAK_HASH", "FQG_TEST_SLOT_CAP", "FQG_NO_PIPELINE")
+HOOKS = ("FQG_MAX_CHUNK_BYTES", "FQG_P2P", "FQG_TEST_WEAK_HASH", "FQG_TEST_SLOT_CAP")
 n = 0
 for nm, rr in (("clean", big), ("dup", dup), ("nul", nul), ("bad", bad)):
     for mode, argv in ((fq.MODE_INDEX, ["a.fq"]), (fq.MODE_SINGLE, ["-r", "a.fq"])):
         for env in ({}, {"FQG_MAX_CHUNK_BYTES": "8192"}, {"FQG_P2P": "1", "FQG_MAX_CHUNK_BYTES": "8192"}, {"FQG_TEST_WEAK_HASH": "1"},
-                    {"FQG_P2P": "1", "FQG_TEST_SLOT_CAP": "5", "FQG_MAX_CHUNK_BYTES": "16384"}, {"FQG_NO_PIPELINE": "1"}):
+                    {"FQG_P2P": "1", "FQG_TEST_SLOT_CAP": "5", "FQG_MAX_CHUNK_BYTES": "16384"}):
             for k in HOOKS:
                 os.environ.pop(k, None)
             os.environ.update(env)

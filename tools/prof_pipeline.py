@@ -1,5 +1,5 @@
 """World-1 run of the pipelined sharded orchestration on synthetic reads: step time and kernel times per class.
-    python tools/prof_pipeline.py [records] ; FQG_NO_PIPELINE=1 for the one-exchange path"""
+    python tools/prof_pipeline.py [records]"""
 import os, sys, time
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 import torch
@@ -33,7 +33,7 @@ for i in range(5):
     torch.cuda.synchronize(); ts.append((time.perf_counter() - t0) * 1e3)
 if dist.is_initialized() and dist.get_rank() != 0:
     sys.exit(0)
-print("pipeline", run.pipeline, "rounds", run.rounds_done, "step ms", [round(x, 2) for x in ts], "GB/s", round(n * rb / min(ts[2:]) / 1e6, 1), "rc", res["transcript"][0], res["n_index_entries"])
+print("rounds", run.rounds_done, "step ms", [round(x, 2) for x in ts], "GB/s", round(n * rb / min(ts[2:]) / 1e6, 1), "rc", res["transcript"][0], res["n_index_entries"])
 for nm, c in (("ctx", run.ctx), ("shard", run.shard)):
     ks = c.kernel_stats()
     print(nm, {k: (round(v["ms"] / 3, 3), v["launches"] // 3) for k, v in ks.items() if v["launches"]})
