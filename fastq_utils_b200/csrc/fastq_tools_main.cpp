@@ -1,11 +1,14 @@
 /*
- * fastq_tools_gpu — the reference's reader- and writer-style command lines on top of libfastq_gpu: fastq_num_reads, fastq_not_empty,
- * fastq_truncate, fastq_filter_n (src/fastq_num_reads.c, src/fastq_not_empty.c, src/fastq_truncate.c, src/fastq_filter_n.c),
- * fastq_trim_poly_at (src/fastq_trim_poly_at.c) and fastq_filterpair (src/fastq_filterpair.c).  One binary: the tool is the name it is
- * called by (symbolic links <tool>_gpu next to it) or, called as fastq_tools_gpu, its first argument.  Same arguments, same stdout /
- * stderr text, same exit status, same output files.  The host inflates the inputs (zlib, like the reference's gzopen / gzgets: gzip
- * members are concatenated, plain text passes through, `-` is standard input), gzips what the writers return with the reference's
- * compression levels, and prints; records are delimited, names indexed and looked up, reads scanned on the GPU.
+ * fastq_tools_gpu — the reference's command lines on top of libfastq_gpu: fastq_info (src/fastq_info.c:190-396), fastq_num_reads,
+ * fastq_not_empty, fastq_truncate, fastq_filter_n (src/fastq_num_reads.c, src/fastq_not_empty.c, src/fastq_truncate.c,
+ * src/fastq_filter_n.c), fastq_trim_poly_at (src/fastq_trim_poly_at.c) and fastq_filterpair (src/fastq_filterpair.c).  One binary: the
+ * tool is the name it is called by (symbolic links <tool>_gpu next to it) or, called as fastq_tools_gpu, its first argument.  Same
+ * arguments, same stdout / stderr text, same exit status, same output files.  The host inflates the inputs (zlib, like the reference's
+ * gzopen / gzgets: gzip members are concatenated, plain text passes through, `-` is standard input), gzips what the writers return with
+ * the reference's compression levels, and prints; every FASTQ byte is checked, records are delimited, names indexed and looked up, reads
+ * scanned on the GPU.  fastq_info streams its files: the library asks for the operands it would open (fqg_fastq_info_stream) and reads
+ * them piece by piece (FQG_PIECE_BYTES, default 64 MiB) through the callbacks below, inflating one piece on a helper thread while the
+ * previous one is copied to the device and validated.
  */
 #include <zlib.h>
 #include <cstdio>
@@ -57,14 +60,20 @@ int main(int argc, char** argv) {
   if (tool.rfind('/') != std::string::npos) tool = tool.substr(tool.rfind('/') + 1);
   if (tool.size() > 4 && tool.compare(tool.size() - 4, 4, "_gpu") == 0) tool.resize(tool.size() - 4);
   if (tool == "fastq_tools") {
-    if (argc < 2) { fprintf(stderr, "usage: fastq_tools_gpu <fastq_num_reads|fastq_not_empty|fastq_truncate|fastq_filter_n|fastq_trim_poly_at|fastq_filterpair> arguments...\n"); return 1; }
+    if (argc < 2) { fprintf(stderr, "usage: fastq_tools_gpu <fastq_info|fastq_num_reads|fastq_not_empty|fastq_truncate|fastq_filter_n|fastq_trim_poly_at|fastq_filterpair> arguments...\n"); return 1; }
     tool = argv[1]; argv++; argc--;
   }
   std::vector<const char*> av(argv, argv + argc);
   av[0] = tool.c_str();
   fqg_transcript t; memset(&t, 0, sizeof t);
+  fqg_stream_io io; io.user = nullptr; io.open = gz_open; io.read = gz_read; io.close = gz_close;
+  if (tool == "fastq_info") {
+    const char* piece = getenv("FQG_PIECE_BYTES");
+    const int st = fqg_fastq_info_stream(argc, av.data(), &io, dev, piece ? (size_t)strtoull(piece, nullptr, 10) : 0, &t);
+    if (st) return failed(st);
+    return finish(t);
+  }
   if (tool == "fastq_trim_poly_at") {
-    fqg_stream_io io; io.user = nullptr; io.open = gz_open; io.read = gz_read; io.close = gz_close;
     char* data = nullptr; size_t n = 0; const char* oname = nullptr;
     const int st = fqg_trim_poly_at_stream(argc, av.data(), &io, dev, &t, &data, &n, &oname);
     if (st) return failed(st);

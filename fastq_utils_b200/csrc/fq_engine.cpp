@@ -24,7 +24,6 @@ static const double kLanesTile = 31744.0;        /* bytes of a tile of the per-l
 static const int kCounters = 12; /* [8] names claimed / [9] mates without a (fresh) partner at the owner (pipelined routing of paired files) */
 
 static uint64_t pow2_at_least(uint64_t x) { uint64_t p = 1; while (p < x) p <<= 1; return p; }
-static int fmt_of_sniff(int s) { return s == FQ_SNIFF_DEFAULT ? FQ_FMT_DEFAULT : s == FQ_SNIFF_CASAVA ? FQ_FMT_CASAVA : FQ_FMT_INT; }
 
 FqEngine::FqEngine(const fqg_config& cfg, FqDevice* dev) : cfg_(cfg), dev_(dev) {
   if (cfg_.mode == FQG_MODE_READER) { reader_ = true; cfg_.mode = FQG_MODE_SINGLE; } /* same chunks, segments, tails and events; only the per-record verdict differs */
@@ -112,10 +111,10 @@ uint64_t FqEngine::step_base(int file) const { return loop_of(file) == FQ_LOOP_M
 FqRecCtx FqEngine::make_ctx(int file) const {
   FqRecCtx cx; memset(&cx, 0, sizeof cx);
   cx.loop = loop_of(file);
-  cx.fmt_key = fmt_of_sniff(f_[file].sniff_fmt);
+  cx.fmt_key = fq_fmt_of_sniff(f_[file].sniff_fmt);
   cx.pe_key = (cfg_.mode == FQG_MODE_INDEX && !(cfg_.flags & FQG_FLAG_PAIRED_NAMES)) ? 0 : 1; /* fastq_info.c:63,112-113,158,290,327 */
   if (cx.loop == FQ_LOOP_MATE) { /* fastq_info.c:345: file-2 records are validated against file 1's state */
-    cx.fmt_val = fmt_of_sniff(f_[0].sniff_fmt); cx.pe_val = 1; cx.space = f_[0].sniff_color;
+    cx.fmt_val = fq_fmt_of_sniff(f_[0].sniff_fmt); cx.pe_val = 1; cx.space = f_[0].sniff_color;
   } else { cx.fmt_val = cx.fmt_key; cx.pe_val = cx.pe_key; cx.space = f_[file].sniff_color; }
   cx.weight = cx.loop == FQ_LOOP_INDEX ? 2 : 1; /* fastq.c:241 + :344 */
   cx.seed = seed_;

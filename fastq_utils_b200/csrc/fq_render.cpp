@@ -1,7 +1,10 @@
 /*
  * fq_render.cpp — turns a finished report into the text and exit status the reference's fastq_info produces
- * (stdout / stderr split, message wording, blank lines: src/fastq_info.c:190-396, src/fastq.h:69-82), and
- * fqg_fastq_info_mem(): main() on inflated streams — option parsing, mode dispatch, feeding, rendering.
+ * (stdout / stderr split, message wording, blank lines: src/fastq_info.c:190-396, src/fastq.h:69-82), and the main() of
+ * each reference tool on inflated streams: fastq_info (fqg_fastq_info_mem / _stream), fastq_num_reads, fastq_not_empty,
+ * fastq_truncate and fastq_filter_n (fqg_reader_tool_mem), fastq_filterpair (fqg_filterpair_mem) and fastq_trim_poly_at
+ * (fqg_trim_poly_at_stream).  They share one skeleton: options through the C library's getopt as the reference parses them,
+ * early exits that only print, and the engines run on a device by on_device(), which turns an exception into a status.
  */
 #include <getopt.h>
 #include <cstdarg>
@@ -16,6 +19,8 @@
 #include <vector>
 #include "fq_engine.h"
 
+FqDevice* fq_default_device(int ordinal); /* fq_abi.cpp (CUDA) or the test stand-in */
+
 namespace {
 
 struct Text {
@@ -23,6 +28,7 @@ struct Text {
   int rc = 0;
   void o(const char* fmt, ...) { va_list ap; va_start(ap, fmt); vput(out, fmt, ap); va_end(ap); }
   void e(const char* fmt, ...) { va_list ap; va_start(ap, fmt); vput(err, fmt, ap); va_end(ap); }
+  void error(const char* fmt, ...) { err += "\nERROR: "; va_list ap; va_start(ap, fmt); vput(err, fmt, ap); va_end(ap); err += "\n"; } /* PRINT_ERROR */
   static void vput(std::string& s, const char* fmt, va_list ap) {
     va_list ap2; va_copy(ap2, ap);
     int k = vsnprintf(nullptr, 0, fmt, ap2); va_end(ap2);
@@ -31,9 +37,42 @@ struct Text {
     s.append(buf.data(), (size_t)k);
   }
 };
-/* PRINT_ERROR, src/fastq.h:69 */
+/* PRINT_ERROR, src/fastq.h:69, around a message that is put together piece by piece */
 #define ERR_BEGIN(t) (t).err += "\nERROR: "
 #define ERR_END(t) (t).err += "\n"
+
+void banner(Text& t) { t.e("fastq_utils %s\n", "0.25.3"); } /* fastq_print_version */
+void mode_line(Text& t, int mode) { /* the line fastq_info prints for a mode that has one, before it reads a file */
+  switch (mode) {
+    case FQG_MODE_INTERLEAVED: t.e("Paired-end interleaved\n"); break;
+    case FQG_MODE_SORTED_PAIR: t.e("-s option used: assuming that reads have the same ordering in both files\n"); break;
+    case FQG_MODE_SINGLE: t.e("Skipping check for duplicated read names\n"); break;
+    default: break;
+  }
+}
+/* the length the caller passes for an input it could not open */
+const size_t UNOPENABLE = (size_t)-1;
+void unable_to_open(Text& t, const char* name) { t.error("Unable to open %s", name); } /* src/fastq.c:651-655 */
+/* the records the reader loop delivered: those before a record without all four lines, else all of them */
+uint64_t records_delivered(const fqg_report& r) { return r.error.code == FQG_E_TRUNC ? r.reads_before_error[0] : r.file[0].n_records; }
+/* fastq_write_entry2stdout (src/fastq.c:81-86): four `%s` of the line buffers, so a line ends at its first NUL */
+void write_record(std::string& out, const char* bytes, const FqLine* l) {
+  for (int i = 0; i < 4; i++) out.append(bytes + l[i].off, strnlen(bytes + l[i].off, l[i].len));
+}
+
+/* The C library's getopt keeps its state in globals: one parse at a time, started over (optind = 0, the GNU way) and silent
+ * (opterr = 0: the tools print their own message).  getopt permutes the words it is given, so it gets a copy of the pointers;
+ * after the loop the options (and a "--") stand in front of the operands, as the reference sees them. */
+std::mutex getopt_mu;
+struct Getopt {
+  std::lock_guard<std::mutex> lk{getopt_mu};
+  std::vector<char*> argv;
+  Getopt(int argc, const char** a) {
+    for (int i = 0; i < argc; i++) argv.push_back(const_cast<char*>(a[i]));
+    argv.push_back(nullptr);
+    optind = 0; opterr = 0;
+  }
+};
 
 const char* qual_range2enc(unsigned int lo, unsigned int hi) { /* fastq_qualRange2enc, src/fastq.c:274-297 */
   static const char* names[] = {"33", "64", "solexa", "33 *", "sanger"};
@@ -151,14 +190,14 @@ void render_run(Text& t, const fqg_report& r, const fqg_render_opts& o, bool f2_
       t.o("Read length: %lu %lu %u\n", 0L, 0L, 0);
       t.rc = 0; return;
     }
-    ERR_BEGIN(t); t.e("No reads found in %s.", n1); ERR_END(t);
+    t.error("No reads found in %s.", n1);
     t.rc = 3; return;
   }
   if (mate_pass) {
     t.e("File %s processed\n", n1);
     t.e("Next file %s\n", n2);
     if (o.name2 == nullptr) { t.rc = FQG_ERR_USAGE; return; }
-    if (f2_unopenable) { ERR_BEGIN(t); t.e("Unable to open %s", n2); ERR_END(t); t.rc = 1; return; } /* src/fastq.c:651-655 */
+    if (f2_unopenable) { unable_to_open(t, n2); t.rc = 1; return; }
     sniff_lines(t, r.file[1]);
     progress(t, r.reads_before_error[1], 1);
     if (failed && e.code != FQG_E_LEFTOVER) { error_text(t, e, n1, n2); return; }
@@ -170,10 +209,8 @@ void render_run(Text& t, const fqg_report& r, const fqg_render_opts& o, bool f2_
   t.e("Number of reads: %lu\n", num_reads1);
   const char* enc = qual_range2enc((unsigned int)f.min_qual, (unsigned int)f.max_qual);
   if (!enc && !o.no_enc_ok) {
-    ERR_BEGIN(t);
-    if (f.max_qual > FQ_MAX_PHRED) t.e("Unable to determine quality encoding - unknown range [%lu,>%u]", (unsigned long)f.min_qual, FQ_MAX_PHRED);
-    else t.e("Unable to determine quality encoding - unknown range [%lu,%lu]", (unsigned long)f.min_qual, (unsigned long)f.max_qual);
-    ERR_END(t);
+    if (f.max_qual > FQ_MAX_PHRED) t.error("Unable to determine quality encoding - unknown range [%lu,>%u]", (unsigned long)f.min_qual, FQ_MAX_PHRED);
+    else t.error("Unable to determine quality encoding - unknown range [%lu,%lu]", (unsigned long)f.min_qual, (unsigned long)f.max_qual);
     t.rc = 3; return;
   }
   t.e("Quality encoding range: %lu %lu\n", (unsigned long)f.min_qual, (unsigned long)f.max_qual);
@@ -199,6 +236,23 @@ void to_transcript(const Text& t, fqg_transcript* tr) {
   tr->out = (char*)malloc(t.out.size() + 1); memcpy(tr->out, t.out.data(), t.out.size()); tr->out[t.out.size()] = 0; tr->out_len = t.out.size();
   tr->err = (char*)malloc(t.err.size() + 1); memcpy(tr->err, t.err.data(), t.err.size()); tr->err[t.err.size()] = 0; tr->err_len = t.err.size();
 }
+/* the tool exits here with status rc: what it printed so far is the whole transcript */
+int stop(Text& t, fqg_transcript* tr, int rc) { t.rc = rc; to_transcript(t, tr); return 0; }
+
+/* body(device) on a device of its own, released after everything body made (its engines), also when body throws.  An exception
+ * becomes the entry point's status, with its message on stderr. */
+template <class Body>
+int on_device(int device, Body body) {
+  try {
+    std::unique_ptr<FqDevice> dev(fq_default_device(device));
+    body(dev.get());
+  } catch (const std::bad_alloc&) { return FQG_ERR_OOM;
+  } catch (const std::exception& ex) {
+    fprintf(stderr, "libfastq_gpu: %s\n", ex.what());
+    return strstr(ex.what(), "CUDA") ? (strstr(ex.what(), "no CUDA") ? FQG_ERR_NO_DEVICE : FQG_ERR_CUDA) : FQG_ERR_INTERNAL;
+  }
+  return 0;
+}
 
 void feed_all(FqEngine& eng, int file, const void* p, size_t n, size_t chunk) {
   if (chunk == 0 || n <= chunk) { eng.feed_host(file, p, n, true); return; }
@@ -217,7 +271,7 @@ struct Source {
 };
 struct MemSource : Source {
   const void* p[2]; size_t n[2]; size_t chunk;
-  bool open(int file, const char*) override { return n[file] != (size_t)-1; }
+  bool open(int file, const char*) override { return n[file] != UNOPENABLE; }
   void feed(FqEngine& eng, int file) override { feed_all(eng, file, p[file], n[file], chunk); }
 };
 /* The caller's reader (zlib in the CLI) fills one pinned buffer on a helper thread while the engine takes the other: inflating,
@@ -265,20 +319,77 @@ struct StreamSource : Source {
   }
 };
 
-int fastq_info_run(int argc, const char** argv_in, Source& src, int device, fqg_transcript* tr);
+int fastq_info_run(int argc, const char** argv_in, Source& src, int device, fqg_transcript* tr) {
+  Text t;
+  bool is_paired = false, is_interleaved = false, is_sorted = false, empty_ok = false, no_enc_ok = false, skip_names = false;
+  int nopt = 0; /* option characters, not words: "-rs" counts 2 */
+  const char *a1, *a2 = nullptr;
+  banner(t);
+  {
+    Getopt g(argc, argv_in);
+    for (int c; (c = getopt(argc, g.argv.data(), "esfrhq")) != -1; ++nopt) {
+      switch (c) {
+        case 'q': no_enc_ok = true; break;
+        case 'e': empty_ok = true; break;
+        case 's': is_sorted = true; break;
+        case 'r': skip_names = true; break;
+        case 'h': usage(t, true); return stop(t, tr, 0);
+        case 'f':
+          t.e("Fixing (-f) enabled: Replacing . by N (creating .fix.gz files)\n");
+          t.error("-f option is no longer valid.");
+          return stop(t, tr, 1);
+        default: t.error("Option -%c invalid", optopt); return stop(t, tr, 1); /* "--help" is the unknown option '-' */
+      }
+    }
+    if (argc - nopt < 2 || argc - nopt > 3) {
+      t.error("Invalid number of arguments");
+      usage(t, false);
+      return stop(t, tr, 1);
+    }
+    a1 = g.argv[1 + nopt];
+    if (argc - nopt == 3) a2 = g.argv[2 + nopt];
+  }
+  if (a2) { is_paired = true; is_interleaved = strncmp(a2, "pe", 2) == 0; }
+
+  fqg_config cfg; memset(&cfg, 0, sizeof cfg); cfg.device = device;
+  if (is_interleaved) cfg.mode = FQG_MODE_INTERLEAVED;
+  else if (is_paired && is_sorted && skip_names) cfg.mode = FQG_MODE_SORTED_PAIR;
+  else if (!is_paired && skip_names) cfg.mode = FQG_MODE_SINGLE;
+  else {
+    cfg.mode = is_paired && !is_sorted ? FQG_MODE_INDEX_PAIR : FQG_MODE_INDEX;
+    if (is_paired) cfg.flags |= FQG_FLAG_PAIRED_NAMES;
+  }
+  mode_line(t, cfg.mode);
+  if (!src.open(0, a1)) { unable_to_open(t, a1); return stop(t, tr, 1); }
+  if (cfg.mode == FQG_MODE_SORTED_PAIR && !src.open(1, a2)) { unable_to_open(t, a2); return stop(t, tr, 1); }
+  fqg_report rep;
+  bool f2_unopenable = false;
+  const int st = on_device(device, [&](FqDevice* dev) {
+      FqEngine eng(cfg, dev);
+      src.feed(eng, 0);
+      if (cfg.mode == FQG_MODE_INDEX_PAIR) {
+        /* the reference opens file 2 only after file 1 was indexed without error and holds reads */
+        fqg_report r1; eng.finish(&r1);
+        bool stop_after_1 = (r1.error.code != FQG_OK && r1.error.file == 0) || r1.n_index_entries == 0;
+        if (!stop_after_1) { if (src.open(1, a2)) src.feed(eng, 1); else f2_unopenable = true; }
+      } else if (cfg.mode == FQG_MODE_SORTED_PAIR) src.feed(eng, 1);
+      eng.finish(&rep);
+  });
+  if (st) return st;
+  fqg_render_opts o; o.empty_ok = empty_ok; o.no_enc_ok = no_enc_ok; o.name1 = a1; o.name2 = a2;
+  render_run(t, rep, o, f2_unopenable);
+  if (t.rc < 0) return t.rc;
+  to_transcript(t, tr);
+  return 0;
+}
 
 }  // namespace
 
 extern "C" int fqg_render(const fqg_report* rep, const fqg_render_opts* opts, fqg_transcript* tr) {
   if (!rep || !opts || !tr) return FQG_ERR_USAGE;
   Text t;
-  t.e("fastq_utils %s\n", "0.25.3");
-  switch (rep->mode) {
-    case FQG_MODE_INTERLEAVED: t.e("Paired-end interleaved\n"); break;
-    case FQG_MODE_SORTED_PAIR: t.e("-s option used: assuming that reads have the same ordering in both files\n"); break;
-    case FQG_MODE_SINGLE: t.e("Skipping check for duplicated read names\n"); break;
-    default: break;
-  }
+  banner(t);
+  mode_line(t, rep->mode);
   render_run(t, *rep, *opts);
   if (t.rc < 0) return t.rc;
   to_transcript(t, tr);
@@ -289,8 +400,6 @@ extern "C" void fqg_transcript_free(fqg_transcript* t) {
   if (!t) return;
   free(t->out); free(t->err); t->out = t->err = nullptr;
 }
-
-FqDevice* fq_default_device(int ordinal); /* fq_abi.cpp (CUDA) or the test stand-in */
 
 extern "C" int fqg_fastq_info_mem(int argc, const char** argv_in, const void* f1, size_t n1, const void* f2, size_t n2,
                                   int device, size_t chunk_bytes, fqg_transcript* tr) {
@@ -303,112 +412,6 @@ extern "C" int fqg_fastq_info_stream(int argc, const char** argv_in, const fqg_s
   StreamSource src; src.io = io; src.piece = piece_bytes ? piece_bytes : ((size_t)64 << 20);
   return fastq_info_run(argc, argv_in, src, device, tr);
 }
-
-namespace {
-int fastq_info_run(int argc, const char** argv_in, Source& src, int device, fqg_transcript* tr) {
-  Text t;
-  bool is_paired = false, is_interleaved = false, is_sorted = false, empty_ok = false, no_enc_ok = false, skip_names = false;
-  int nopt = 0;
-  t.e("fastq_utils %s\n", "0.25.3");
-  /* getopt("esfrhq") as GNU libc runs it: option words are permuted to the front, in order; "--" ends them */
-  std::vector<const char*> argv; argv.push_back(argc > 0 ? argv_in[0] : "fastq_info");
-  {
-    bool stop = false;
-    for (int i = 1; i < argc; i++) {
-      const char* w = argv_in[i];
-      if (!stop && !strcmp(w, "--")) { argv.push_back(w); stop = true; continue; }
-      if (!stop && w[0] == '-' && w[1] != '\0') argv.push_back(w);
-    }
-    size_t nflag_words = argv.size();
-    stop = false;
-    for (int i = 1; i < argc; i++) {
-      const char* w = argv_in[i];
-      if (!stop && !strcmp(w, "--")) { stop = true; continue; }
-      if (stop || !(w[0] == '-' && w[1] != '\0')) argv.push_back(w);
-    }
-    for (size_t i = 1; i < nflag_words; i++) {
-      const char* w = argv[i];
-      if (!strcmp(w, "--")) break;
-      for (const char* c = w + 1; *c; c++) {
-        switch (*c) {
-          case 'q': no_enc_ok = true; ++nopt; break;
-          case 'e': empty_ok = true; ++nopt; break;
-          case 's': is_sorted = true; ++nopt; break;
-          case 'r': skip_names = true; ++nopt; break;
-          case 'h': usage(t, true); t.rc = 0; to_transcript(t, tr); return 0;
-          case 'f':
-            t.e("Fixing (-f) enabled: Replacing . by N (creating .fix.gz files)\n");
-            ERR_BEGIN(t); t.e("-f option is no longer valid."); ERR_END(t);
-            t.rc = 1; to_transcript(t, tr); return 0;
-          default:
-            ++nopt;
-            ERR_BEGIN(t); t.e("Option -%c invalid", *c); ERR_END(t);
-            t.rc = 1; to_transcript(t, tr); return 0;
-        }
-      }
-    }
-  }
-  if (argc - nopt < 2 || argc - nopt > 3) {
-    ERR_BEGIN(t); t.e("Invalid number of arguments"); ERR_END(t);
-    usage(t, false);
-    t.rc = 1; to_transcript(t, tr); return 0;
-  }
-  const char* a1 = argv[1 + nopt];
-  const char* a2 = (argc - nopt == 3) ? argv[2 + nopt] : nullptr;
-  if (a2) { is_paired = true; is_interleaved = strncmp(a2, "pe", 2) == 0; }
-
-  auto unopenable = [&](const char* name) { ERR_BEGIN(t); t.e("Unable to open %s", name); ERR_END(t); t.rc = 1; to_transcript(t, tr); return 0; };
-  fqg_config cfg; memset(&cfg, 0, sizeof cfg); cfg.device = device;
-  bool second_file = false, f2_unopenable = false;
-  if (is_interleaved) {
-    cfg.mode = FQG_MODE_INTERLEAVED; t.e("Paired-end interleaved\n");
-    if (!src.open(0, a1)) return unopenable(a1);
-  } else if (is_paired && is_sorted && skip_names) {
-    cfg.mode = FQG_MODE_SORTED_PAIR; second_file = true;
-    t.e("-s option used: assuming that reads have the same ordering in both files\n");
-    if (!src.open(0, a1)) return unopenable(a1);
-    if (!src.open(1, a2)) return unopenable(a2);
-  } else if (!is_paired && skip_names) {
-    cfg.mode = FQG_MODE_SINGLE; t.e("Skipping check for duplicated read names\n");
-    if (!src.open(0, a1)) return unopenable(a1);
-  } else {
-    second_file = is_paired && !is_sorted;
-    cfg.mode = second_file ? FQG_MODE_INDEX_PAIR : FQG_MODE_INDEX;
-    if (is_paired) cfg.flags |= FQG_FLAG_PAIRED_NAMES;
-    if (!src.open(0, a1)) return unopenable(a1);
-  }
-  fqg_report rep;
-  try {
-    std::unique_ptr<FqDevice> dev_owner(fq_default_device(device)); /* released after the engines, also when one of them throws */
-    FqDevice* dev = dev_owner.get();
-    {
-      FqEngine eng(cfg, dev);
-      src.feed(eng, 0);
-      if (second_file) {
-        bool open2 = true;
-        if (cfg.mode == FQG_MODE_INDEX_PAIR) {
-          /* the reference opens file 2 only after file 1 was indexed without error and holds reads */
-          fqg_report r1; eng.finish(&r1);
-          bool stop_after_1 = (r1.error.code != FQG_OK && r1.error.file == 0) || r1.n_index_entries == 0;
-          if (stop_after_1) open2 = false;
-          else if (!src.open(1, a2)) { open2 = false; f2_unopenable = true; }
-        }
-        if (open2) src.feed(eng, 1);
-      }
-      eng.finish(&rep);
-    }
-  } catch (const std::bad_alloc&) { return FQG_ERR_OOM;
-  } catch (const std::exception& ex) {
-    fprintf(stderr, "libfastq_gpu: %s\n", ex.what());
-    return strstr(ex.what(), "CUDA") ? (strstr(ex.what(), "no CUDA") ? FQG_ERR_NO_DEVICE : FQG_ERR_CUDA) : FQG_ERR_INTERNAL;
-  }
-  fqg_render_opts o; o.empty_ok = empty_ok; o.no_enc_ok = no_enc_ok; o.name1 = a1; o.name2 = a2;
-  render_run(t, rep, o, f2_unopenable);
-  if (t.rc < 0) return t.rc;
-  to_transcript(t, tr);
-  return 0;
-}
-}  // namespace
 
 namespace {
 /* main() of the reader tools that WRITE records: src/fastq_truncate.c:32-57 (the first num_reads entries) and src/fastq_filter_n.c:33-93
@@ -438,8 +441,8 @@ WindowsResult reader_windows(FqDevice* dev, int device, const char* p, size_t n,
     FqEngine eng(cfg, dev);
     eng.feed_host(0, p + pos, len, true);
     fqg_report rep; eng.finish(&rep);
-    const bool trunc = rep.error.code == FQG_E_TRUNC; /* the loop met a record without all four lines ... */
-    uint64_t nrec = trunc ? rep.reads_before_error[0] : rep.file[0].n_records; /* ... after this many entries (else: all that fastq_read_entry delivered) */
+    const bool trunc = rep.error.code == FQG_E_TRUNC; /* the loop met a record without all four lines */
+    uint64_t nrec = records_delivered(rep);
     const bool cut_line = !final && len > 0 && p[pos + len - 1] != '\n';
     if (!final && !trunc && cut_line && nrec > 0) nrec--; /* its fourth line is where the window was cut */
     if (!final && nrec == 0 && (trunc || cut_line)) {
@@ -466,46 +469,27 @@ WindowsResult reader_windows(FqDevice* dev, int device, const char* p, size_t n,
 }
 
 int writer_tool(bool filter_n, int argc, const char** argv_in, const void* f1, size_t n1, int device, fqg_transcript* tr) {
-  const size_t UNOPENABLE = (size_t)-1;
   Text t;
-  t.e("fastq_utils %s\n", "0.25.3");
+  banner(t);
   const char* fname = nullptr; long num_reads = 0; unsigned max_n = 0;
   if (!filter_n) {
-    if (argc != 3) { t.e("Usage: fastq_truncate fastq1 num_reads\n"); t.rc = 1; to_transcript(t, tr); return 0; }
+    if (argc != 3) { t.e("Usage: fastq_truncate fastq1 num_reads\n"); return stop(t, tr, 1); }
     fname = argv_in[1]; num_reads = atol(argv_in[2]);
   } else {
-    /* getopt(argc, argv, "n:") with opterr = 0, as GNU libc runs it: option words (and the arguments they take) are permuted to the front */
-    std::vector<const char*> opts, rest; int nopt = 0;
-    bool stop = false;
-    for (int i = 1; i < argc; i++) {
-      const char* w = argv_in[i];
-      if (!stop && !strcmp(w, "--")) { opts.push_back(w); stop = true; continue; }
-      if (stop || !(w[0] == '-' && w[1] != '\0')) { rest.push_back(w); continue; }
-      opts.push_back(w);
-      for (const char* c = w + 1; *c; c++) {
-        if (*c == 'n') {
-          const char* arg = c[1] ? c + 1 : (i + 1 < argc ? argv_in[++i] : nullptr);
-          if (!arg) { ++nopt; ERR_BEGIN(t); t.e("Option -%c invalid", 'n'); ERR_END(t); t.rc = 1; to_transcript(t, tr); return 0; } /* a missing argument is getopt's '?' */
-          if (!c[1]) opts.push_back(arg);
-          max_n = (unsigned)atoi(arg); if (max_n > 100) max_n = 100;
-          nopt += 2;
-          break; /* the rest of the word was the argument */
-        }
-        ++nopt; ERR_BEGIN(t); t.e("Option -%c invalid", *c); ERR_END(t); t.rc = 1; to_transcript(t, tr); return 0;
-      }
+    Getopt g(argc, argv_in);
+    int nopt = 0;
+    for (int c; (c = getopt(argc, g.argv.data(), "n:")) != -1;) {
+      if (c != 'n') { t.error("Option -%c invalid", optopt); return stop(t, tr, 1); } /* "-n" without its argument too */
+      max_n = (unsigned)atoi(optarg); if (max_n > 100) max_n = 100;
+      nopt += 2; /* also for "-n10" */
     }
-    if (argc - nopt < 2 || argc - nopt > 3) { ERR_BEGIN(t); t.e("Usage: fastq_filter_n [ -n 0 ] fastq1"); ERR_END(t); t.rc = 1; to_transcript(t, tr); return 0; }
-    std::vector<const char*> argv; argv.push_back(argv_in[0]);
-    argv.insert(argv.end(), opts.begin(), opts.end()); argv.insert(argv.end(), rest.begin(), rest.end());
+    if (argc - nopt < 2 || argc - nopt > 3) { t.error("Usage: fastq_filter_n [ -n 0 ] fastq1"); return stop(t, tr, 1); }
     if (max_n > 0) t.e("Discard reads with more than %d%% of Ns\n", (int)max_n); else t.e("Discard reads with at least one N\n");
-    fname = (size_t)(nopt + 1) < argv.size() ? argv[nopt + 1] : "";
+    fname = g.argv[nopt + 1];
   }
-  if (n1 == UNOPENABLE) { ERR_BEGIN(t); t.e("Unable to open %s", fname); ERR_END(t); t.rc = 1; to_transcript(t, tr); return 0; }
+  if (n1 == UNOPENABLE) { unable_to_open(t, fname); return stop(t, tr, 1); }
   if (!f1 && n1) return FQG_ERR_USAGE;
-  try {
-    std::unique_ptr<FqDevice> dev_owner(fq_default_device(device)); /* released after the engines, also when one of them throws */
-    FqDevice* dev = dev_owner.get();
-    {
+  const int st = on_device(device, [&](FqDevice* dev) {
       const uint64_t want = (filter_n || num_reads < 0) ? ~0ull : (uint64_t)num_reads;
       WindowsResult W = reader_windows(dev, device, (const char*)f1, n1, want, [&](FqEngine& eng, const std::vector<FqLine>& L, const uint8_t* ddata, const char* bytes, uint64_t g0) {
         std::vector<uint32_t> nn;
@@ -519,22 +503,18 @@ int writer_tool(bool filter_n, int argc, const char** argv_in, const void* f1, s
             const unsigned long read_len = nn[2 * r + 1];
             const unsigned max_num_n = (unsigned)(read_len * max_n / 100);
             const bool keep = nn[2 * r] <= max_num_n;
-            if (keep) for (int i = 0; i < 4; i++) { const FqLine& l = L[4 * r + i]; t.out.append(bytes + l.off, strnlen(bytes + l.off, l.len)); }
+            if (keep) write_record(t.out, bytes, &L[4 * r]);
             const unsigned long cline = 4ul * (unsigned long)(g0 + r + 1);
             if (cline % 100000 == 0) t.e("\b\b\b\b\b\b\b\b\b\b\b\b\b\b\b%lu", cline);
-          } else for (int i = 0; i < 4; i++) { const FqLine& l = L[4 * r + i]; t.out.append(bytes + l.off, strnlen(bytes + l.off, l.len)); }
+          } else write_record(t.out, bytes, &L[4 * r]);
         }
         return true;
       });
       /* the loop met the broken record only if it went on reading that far (src/fastq_truncate.c:47-49) */
       if (W.truncated) { error_text(t, W.error, fname, fname); t.rc = 1; }
       else t.rc = 0;
-    }
-  } catch (const std::bad_alloc&) { return FQG_ERR_OOM;
-  } catch (const std::exception& ex) {
-    fprintf(stderr, "libfastq_gpu: %s\n", ex.what());
-    return strstr(ex.what(), "CUDA") ? (strstr(ex.what(), "no CUDA") ? FQG_ERR_NO_DEVICE : FQG_ERR_CUDA) : FQG_ERR_INTERNAL;
-  }
+  });
+  if (st) return st;
   to_transcript(t, tr);
   return 0;
 }
@@ -555,13 +535,13 @@ struct PairFile { /* one input: its records (reader loop) on the device and on t
     rd = new FqEngine(cfg, dev);
     rd->feed_host(0, p, n, true);
     rd->finish(&rep);
-    nrec = rep.error.code == FQG_E_TRUNC ? rep.reads_before_error[0] : rep.file[0].n_records;
+    nrec = records_delivered(rep);
     rd->record_table(nrec, &L, &ddata);
     bytes = (const char*)p;
   }
   ~PairFile() { delete rd; }
   std::vector<FqLine> headers() const { std::vector<FqLine> h(L.size() / 4); for (size_t r = 0; r < h.size(); r++) h[r] = L[4 * r]; return h; }
-  void write(std::string& out, size_t r) const { for (int i = 0; i < 4; i++) { const FqLine& l = L[4 * r + i]; out.append(bytes + l.off, strnlen(bytes + l.off, l.len)); } }
+  void write(std::string& out, size_t r) const { write_record(out, bytes, &L[4 * r]); }
   uint32_t raw_len(size_t r) const { return L[4 * r].len + L[4 * r + 1].len + L[4 * r + 2].len + L[4 * r + 3].len; }
 };
 /* the index loop over one file (fastq_index_readnames and the lines fastq_filterpair prints around it); false: it ended the run */
@@ -582,15 +562,14 @@ bool index_file(Text& t, FqEngine& ix, const void* p, size_t n, const char* name
 extern "C" int fqg_filterpair_mem(int argc, const char** argv, const void* f1, size_t n1, const void* f2, size_t n2, int device,
                                   fqg_transcript* tr, char* outs[3], size_t lens[3], int32_t* created) {
   if (argc < 1 || !argv || !tr || !outs || !lens || !created) return FQG_ERR_USAGE;
-  const size_t UNOPENABLE = (size_t)-1;
   for (int i = 0; i < 3; i++) { outs[i] = nullptr; lens[i] = 0; }
   *created = 0;
   Text t;
-  t.e("fastq_utils %s\n", "0.25.3");
-  if (argc != 6 && argc != 7) { t.e("Usage: filterpair fastq1 fastq2 paired1 paired2 unpaired [sorted]\n"); t.rc = 1; to_transcript(t, tr); return 0; }
+  banner(t);
+  if (argc != 6 && argc != 7) { t.e("Usage: filterpair fastq1 fastq2 paired1 paired2 unpaired [sorted]\n"); return stop(t, tr, 1); }
   t.e("%d", argc);
-  if (n1 == UNOPENABLE) { ERR_BEGIN(t); t.e("Unable to open %s", argv[1]); ERR_END(t); t.rc = 1; to_transcript(t, tr); return 0; } /* src/fastq.c:651-655 */
-  if (n2 == UNOPENABLE) { ERR_BEGIN(t); t.e("Unable to open %s", argv[2]); ERR_END(t); t.rc = 1; to_transcript(t, tr); return 0; }
+  if (n1 == UNOPENABLE) { unable_to_open(t, argv[1]); return stop(t, tr, 1); }
+  if (n2 == UNOPENABLE) { unable_to_open(t, argv[2]); return stop(t, tr, 1); }
   if ((!f1 && n1) || (!f2 && n2)) return FQG_ERR_USAGE;
   const size_t LIMIT = ((size_t)1 << 31) - 64; /* one chunk per file: the record-writing tools take streams below 2 GiB */
   if (n1 > LIMIT || n2 > LIMIT) return FQG_ERR_USAGE;
@@ -599,10 +578,7 @@ extern "C" int fqg_filterpair_mem(int argc, const char** argv, const void* f1, s
   if (sorted) t.e("Assuming sorted fastq files\n");
   std::string out[3]; /* paired1, paired2, unpaired */
   fqg_config cfg; memset(&cfg, 0, sizeof cfg); cfg.device = device; cfg.mode = FQG_MODE_INDEX; cfg.flags = FQG_FLAG_PAIRED_NAMES;
-  try {
-    std::unique_ptr<FqDevice> dev_owner(fq_default_device(device)); /* released after the engines, also when one of them throws */
-    FqDevice* dev = dev_owner.get();
-    {
+  const int st = on_device(device, [&](FqDevice* dev) {
       unsigned long index_mem = 0;
       fqg_report rep1, rep2;
       FqEngine ix1(cfg, dev);
@@ -611,14 +587,14 @@ extern "C" int fqg_filterpair_mem(int argc, const char** argv, const void* f1, s
         *created = 1; /* the three output files exist from here on (src/fastq_filterpair.c:83-92) */
         PairFile A, B;
         A.load(cfg, dev, f1, n1);
-        const int fmt1 = rep1.file[0].sniff_format == FQ_SNIFF_DEFAULT ? FQ_FMT_DEFAULT : rep1.file[0].sniff_format == FQ_SNIFF_CASAVA ? FQ_FMT_CASAVA : FQ_FMT_INT;
+        const int fmt1 = fq_fmt_of_sniff(rep1.file[0].sniff_format);
         unsigned long paired = 0, up2 = 0;
         if (sorted) {
           FqEngine ix2(cfg, dev);
           go = index_file(t, ix2, f2, n2, argv[2], &index_mem, &rep2);
           if (go) {
             B.load(cfg, dev, f2, n2);
-            const int fmt2 = rep2.file[0].sniff_format == FQ_SNIFF_DEFAULT ? FQ_FMT_DEFAULT : rep2.file[0].sniff_format == FQ_SNIFF_CASAVA ? FQ_FMT_CASAVA : FQ_FMT_INT;
+            const int fmt2 = fq_fmt_of_sniff(rep2.file[0].sniff_format);
             /* both files hold every name once (the index loop saw to that): a record has its mate iff the other index holds its name */
             std::vector<unsigned long long> in2, in1;
             FqName* na = ix2.header_names(A.ddata, A.headers(), fmt1, 1);
@@ -645,7 +621,7 @@ extern "C" int fqg_filterpair_mem(int argc, const char** argv, const void* f1, s
           std::vector<unsigned long long> hit; std::vector<FqName> names2;
           if (B.nrec) {
             B.rd->sniff_first(B.ddata, B.L[0], B.L[1], &sf2, &col2);
-            const int fmt2 = sf2 == FQ_SNIFF_DEFAULT ? FQ_FMT_DEFAULT : sf2 == FQ_SNIFF_CASAVA ? FQ_FMT_CASAVA : FQ_FMT_INT;
+            const int fmt2 = fq_fmt_of_sniff(sf2);
             FqName* nb = ix1.header_names(B.ddata, B.headers(), fmt2, 1);
             ix1.lookup_names(nb, B.ddata, (uint32_t)B.nrec, &hit);
             names2.resize(B.nrec);
@@ -698,12 +674,8 @@ extern "C" int fqg_filterpair_mem(int argc, const char** argv, const void* f1, s
           if (paired == 0) { t.e("!!!WARNING!!! 0 paired reads! are the headers ok?\n"); t.rc = 3; } else t.rc = 0;
         }
       }
-    }
-  } catch (const std::bad_alloc&) { return FQG_ERR_OOM;
-  } catch (const std::exception& ex) {
-    fprintf(stderr, "libfastq_gpu: %s\n", ex.what());
-    return strstr(ex.what(), "CUDA") ? (strstr(ex.what(), "no CUDA") ? FQG_ERR_NO_DEVICE : FQG_ERR_CUDA) : FQG_ERR_INTERNAL;
-  }
+  });
+  if (st) return st;
   for (int i = 0; i < 3; i++) {
     outs[i] = (char*)malloc(out[i].size() + 1);
     if (!outs[i]) return FQG_ERR_OOM;
@@ -727,21 +699,12 @@ extern "C" int fqg_trim_poly_at_stream(int argc, const char** argv_in, const fqg
   *outfile = nullptr; *outfile_len = 0; *outfile_name = nullptr;
   Text t;
   const char* file = nullptr; const char* ofile = nullptr; int min_poly = 10; long min_len = 10;
-  static std::mutex getopt_mu; /* getopt's state is the C library's: one parse at a time */
   int help = 0;
   {
-    std::lock_guard<std::mutex> lk(getopt_mu);
-    static int help_flag; help_flag = 0;
-    static struct option long_options[] = {{"help", no_argument, &help_flag, 1}, {"min_poly_at_len", required_argument, 0, 'a'}, {"file", required_argument, 0, 'b'},
-                                           {"outfile", required_argument, 0, 'c'}, {"min_len", required_argument, 0, 'd'}, {0, 0, 0, 0}};
-    std::vector<char*> argv; /* getopt permutes the words: a copy of the pointers */
-    for (int i = 0; i < argc; i++) argv.push_back(const_cast<char*>(argv_in[i]));
-    argv.push_back(nullptr);
-    optind = 0; opterr = 0; /* (optind = 0: the GNU way to start over) */
-    for (;;) {
-      int option_index = 0;
-      const int c = getopt_long(argc, argv.data(), "a:b:c:d:", long_options, &option_index);
-      if (c == -1) break;
+    const struct option long_options[] = {{"help", no_argument, &help, 1}, {"min_poly_at_len", required_argument, 0, 'a'}, {"file", required_argument, 0, 'b'},
+                                          {"outfile", required_argument, 0, 'c'}, {"min_len", required_argument, 0, 'd'}, {0, 0, 0, 0}};
+    Getopt g(argc, argv_in);
+    for (int c; (c = getopt_long(argc, g.argv.data(), "a:b:c:d:", long_options, nullptr)) != -1;) {
       switch (c) {
         case 'a': min_poly = (int)atol(optarg); break;
         case 'b': file = optarg; break;
@@ -750,21 +713,20 @@ extern "C" int fqg_trim_poly_at_stream(int argc, const char** argv_in, const fqg
         default: break;
       }
     }
-    help = help_flag;
   }
-  t.e("fastq_utils %s\n", "0.25.3");
+  banner(t);
   if (help) {
     t.o("usage: fastq_trim_poly_at --file fastq_file --outfile out_file [optional parameters]");
     t.o("%s", "\n  --help       :print the usage\n  --file <filename> :fastq (optional gzipped) file name \n  --ofile <filename> : fastq file name where the processed reads will be written \n"
               "  --min_poly_at_len integer     : minimum length of poly-A|T sequence to remove.\n  --min_len integer     : minimum read length.\n");
-    t.rc = 0; to_transcript(t, tr); return 0;
+    return stop(t, tr, 0);
   }
   t.e("INFO:Validating options...\n");
-  if (!file) { ERR_BEGIN(t); t.e("missing input file (--file)"); ERR_END(t); t.rc = 1; to_transcript(t, tr); return 0; }
-  if (!ofile) { ERR_BEGIN(t); t.e("missing output file name (--outfile)"); ERR_END(t); t.rc = 1; to_transcript(t, tr); return 0; }
+  if (!file) { t.error("missing input file (--file)"); return stop(t, tr, 1); }
+  if (!ofile) { t.error("missing output file name (--outfile)"); return stop(t, tr, 1); }
   t.e("INFO:Options OK.\n");
   void* h = io->open ? io->open(io->user, file) : nullptr;
-  if (!h) { ERR_BEGIN(t); t.e("Unable to open %s", file); ERR_END(t); t.rc = 1; to_transcript(t, tr); return 0; } /* src/fastq.c:651-655 */
+  if (!h) { unable_to_open(t, file); return stop(t, tr, 1); }
   std::vector<char> in;
   {
     std::vector<char> piece(8u << 20);
@@ -775,10 +737,7 @@ extern "C" int fqg_trim_poly_at_stream(int argc, const char** argv_in, const fqg
   }
   *outfile_name = ofile; /* from here on the reference has created the file */
   std::string out;
-  try {
-    std::unique_ptr<FqDevice> dev_owner(fq_default_device(device)); /* released after the engines, also when one of them throws */
-    FqDevice* dev = dev_owner.get();
-    {
+  const int st = on_device(device, [&](FqDevice* dev) {
       std::vector<char> sbuf(4, 0), qbuf(4, 0); /* the entry's seq and qual buffers: they outlive a record (and a window) */
       unsigned long trimmed = 0, discarded = 0, processed = 0;
       WindowsResult W = reader_windows(dev, device, in.data(), in.size(), ~0ull, [&](FqEngine& eng, const std::vector<FqLine>& L, const uint8_t* ddata, const char* bytes, uint64_t g0) {
@@ -823,12 +782,8 @@ extern "C" int fqg_trim_poly_at_stream(int argc, const char** argv_in, const fqg
         t.e("INFO:Reads processed: %ld\n", (long)processed); t.e("INFO:Reads trimmed: %ld\n", (long)trimmed); t.e("INFO:Reads discarded: %ld\n", (long)discarded);
         t.rc = 0;
       }
-    }
-  } catch (const std::bad_alloc&) { return FQG_ERR_OOM;
-  } catch (const std::exception& ex) {
-    fprintf(stderr, "libfastq_gpu: %s\n", ex.what());
-    return strstr(ex.what(), "CUDA") ? (strstr(ex.what(), "no CUDA") ? FQG_ERR_NO_DEVICE : FQG_ERR_CUDA) : FQG_ERR_INTERNAL;
-  }
+  });
+  if (st) return st;
   *outfile = (char*)malloc(out.size() + 1);
   if (!*outfile) return FQG_ERR_OOM;
   memcpy(*outfile, out.data(), out.size()); (*outfile)[out.size()] = 0; *outfile_len = out.size();
@@ -842,35 +797,27 @@ extern "C" void fqg_buffer_free(void* p) { free(p); }
  * a record with fewer than four lines is "file truncated" (exit 1); nothing is validated. */
 extern "C" int fqg_reader_tool_mem(int argc, const char** argv, const void* f1, size_t n1, int device, size_t chunk_bytes, fqg_transcript* tr) {
   if (argc < 1 || !argv || !argv[0] || !tr) return FQG_ERR_USAGE;
-  const size_t UNOPENABLE = (size_t)-1;
   Text t;
   const char* tool = strrchr(argv[0], '/'); tool = tool ? tool + 1 : argv[0];
   const bool num_reads = !strcmp(tool, "fastq_num_reads"), not_empty = !strcmp(tool, "fastq_not_empty");
   if (!strcmp(tool, "fastq_truncate") || !strcmp(tool, "fastq_filter_n")) return writer_tool(!strcmp(tool, "fastq_filter_n"), argc, argv, f1, n1, device, tr);
   if (!num_reads && !not_empty) return FQG_ERR_USAGE;
-  if (num_reads) t.e("fastq_utils %s\n", "0.25.3"); /* fastq_print_version, src/fastq_num_reads.c:34; fastq_not_empty prints none */
+  if (num_reads) banner(t); /* src/fastq_num_reads.c:34; fastq_not_empty prints none */
   if (argc != 2) {
-    if (num_reads) { t.e("Usage: fastq_num_reads fastq_file\n"); t.rc = 1; }
-    else { t.e("Usage: fastq_not_empty fastq_file\nExit status of 0 if it is not empty, 0 otherwise. The fastq file may be compressed with gzip."); t.rc = 1; }
-    to_transcript(t, tr); return 0;
+    if (num_reads) t.e("Usage: fastq_num_reads fastq_file\n");
+    else t.e("Usage: fastq_not_empty fastq_file\nExit status of 0 if it is not empty, 0 otherwise. The fastq file may be compressed with gzip.");
+    return stop(t, tr, 1);
   }
-  if (n1 == UNOPENABLE) { ERR_BEGIN(t); t.e("Unable to open %s", argv[1]); ERR_END(t); t.rc = 1; to_transcript(t, tr); return 0; } /* src/fastq.c:651-655 */
+  if (n1 == UNOPENABLE) { unable_to_open(t, argv[1]); return stop(t, tr, 1); }
   if (!f1 && n1) return FQG_ERR_USAGE;
   fqg_config cfg; memset(&cfg, 0, sizeof cfg); cfg.device = device; cfg.mode = FQG_MODE_READER;
   fqg_report rep;
-  try {
-    std::unique_ptr<FqDevice> dev_owner(fq_default_device(device)); /* released after the engines, also when one of them throws */
-    FqDevice* dev = dev_owner.get();
-    {
+  const int st = on_device(device, [&](FqDevice* dev) {
       FqEngine eng(cfg, dev);
       feed_all(eng, 0, f1, n1, chunk_bytes);
       eng.finish(&rep);
-    }
-  } catch (const std::bad_alloc&) { return FQG_ERR_OOM;
-  } catch (const std::exception& ex) {
-    fprintf(stderr, "libfastq_gpu: %s\n", ex.what());
-    return strstr(ex.what(), "CUDA") ? (strstr(ex.what(), "no CUDA") ? FQG_ERR_NO_DEVICE : FQG_ERR_CUDA) : FQG_ERR_INTERNAL;
-  }
+  });
+  if (st) return st;
   const uint64_t n = rep.file[0].n_records;
   if (not_empty) { /* only the first entry is ever read: an error further down does not exist for this tool */
     if (rep.reads_before_error[0] >= 1) t.rc = 0;

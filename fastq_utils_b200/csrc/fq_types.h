@@ -25,6 +25,8 @@
 enum { FQ_FMT_UNDEF = -1, FQ_FMT_DEFAULT = 0, FQ_FMT_CASAVA = 1, FQ_FMT_INT = 2 };
 /* what the format sniff found (decides which info line is printed, src/fastq.c:459-478) */
 enum { FQ_SNIFF_DEFAULT = 0, FQ_SNIFF_CASAVA = 1, FQ_SNIFF_INT = 2, FQ_SNIFF_NOSUFFIX = 3 };
+/* the read-name format a file's sniff selects */
+FQ_HD int fq_fmt_of_sniff(int s) { return s == FQ_SNIFF_DEFAULT ? FQ_FMT_DEFAULT : s == FQ_SNIFF_CASAVA ? FQ_FMT_CASAVA : FQ_FMT_INT; }
 enum { FQ_SPACE_UNDEF = -1, FQ_SPACE_SEQ = 0, FQ_SPACE_COLOR = 1 };
 
 /* per-record validation outcome: the first failing step of fastq_validate_entry (src/fastq.c:300-392) */
